@@ -2,6 +2,7 @@
 """bench.py -- converged IK solves/sec on the BASELINE.json headline workload.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dtype f64|f32] [--batch B]
+                    [--dump-outputs DIR]
 
 Workload (`config`, identical in both arms): Cassie feet+pelvis IK (pelvis Full + LeftFootFront / RightFootFront
 Position, world frame), library-default solver parameters (max_iterations 100, damping 1e-2, step 1.0), batch 65,536
@@ -29,12 +30,17 @@ A "step" = one batched ik::dls over one batch of B problems.
   strong    the SAME global batch (65,536 Cassie; 1,048,576 manipulator) cut over the N ranks (SURVEY 8e).
   cpu_baseline / --impl reference: the restated reference CPU path (oracle/, "port": Pinocchio / Eigen are unavailable so
             the reference itself cannot be built), all host cores; that arm imports nothing from the product.
+
+--dump-outputs DIR writes what the headline path returned for its last timed step (rank 0's batch) as DIR/<name>.npy:
+q (nq x B), success, iters and resid, all in the solve's float type.  The inputs are seeded, so two builds run with the
+same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
 import json
 import os
 import sys
+import tempfile
 import threading
 import time
 
@@ -62,6 +68,25 @@ def static_config(batch, world, dtype):
 def hbm_bytes_per_solve(nq, tsz, s):
     # (q0 + targets) in, (q + resid) + success(1) + iters(4) out -- SURVEY 8d "Layout"
     return (nq + tsz) * s + (nq + 1) * s + 1 + 4
+
+
+DUMP_LIMIT_BYTES = 63 << 20   # array data of --dump-outputs: with the .npy headers, under 64 MB in all
+
+
+def dump_outputs(out_dir, outputs, dtype):
+    """Writes each output array (batch along the last axis) as <out_dir>/<name>.npy in `dtype`.  When they exceed
+    DUMP_LIMIT_BYTES, a fixed, seeded sample of problems is written instead, with their batch indices in index.npy."""
+    arrays = {k: np.asarray(v).astype(dtype) for k, v in outputs.items()}
+    B = arrays["success"].shape[-1]
+    per_problem = sum(a.nbytes for a in arrays.values()) // B
+    if per_problem * B > DUMP_LIMIT_BYTES:
+        n = DUMP_LIMIT_BYTES // (per_problem + 8)
+        idx = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+        arrays = {k: a[..., idx] for k, a in arrays.items()}
+        arrays["index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def f_iter(model, pb):
@@ -184,7 +209,11 @@ def main():
     ap.add_argument("--e2e-merge", type=int, default=4, help="the same for the host-buffer (e2e) arm: smaller groups keep the "
                     "PCIe pipeline's fill / drain short")
     ap.add_argument("--e2e-depth", type=int, default=12, help="three groups in flight: host batches carry their stragglers too (ikb_queue_create)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write q, success, iters and resid of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -341,6 +370,10 @@ def main():
     launches = ik.kernel_launch_count() - launches0
     elapsed_ms = ev[0].elapsed_time(ev[1])
     sampler.armed.clear()
+    # the later sections reuse these output buffers
+    last_outputs = None
+    if args.dump_outputs and rank == 0:
+        last_outputs = {k: v.cpu().numpy() for k, v in sets[(args.steps - 1) % nsets][2].items()}
 
     # optional final result gather (SURVEY 8e): not part of the solve, timed and reported separately
     gather_ms = None
@@ -593,7 +626,7 @@ def main():
         # several GPUs through the PRODUCT (ikb_multi_*): one host thread on rank 0 shards a host batch of world x B problems
         # over all visible GPUs.  The other ranks must leave their GPUs idle meanwhile -- an NCCL barrier would keep a
         # spinning kernel on each of them -- so they wait on a file flag, on the CPU.
-        flag = "/tmp/ikb_bench_multi_done_%s" % os.environ.get("MASTER_PORT", "0")
+        flag = os.path.join(tempfile.gettempdir(), "ikb_bench_multi_done_%d_%s" % (os.getuid(), os.environ.get("MASTER_PORT", "0")))
         if rank == 0 and os.path.exists(flag):
             os.remove(flag)
         barrier()
@@ -635,6 +668,8 @@ def main():
             while not os.path.exists(flag) and time.time() - t_wait < 300:
                 time.sleep(0.01)
         barrier()
+        if rank == 0:
+            os.remove(flag)
 
     # ---- reduce over ranks ----
     stats = torch.tensor([elapsed_ms, e2e_s, full_s], dtype=torch.float64, device=dev)
@@ -728,6 +763,8 @@ def main():
             "product_multi_gpu": product_multi,
             "clocks": sampler.summary(),
         }
+        if last_outputs is not None:
+            dump_outputs(args.dump_outputs, last_outputs, npdt)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

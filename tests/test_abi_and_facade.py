@@ -6,6 +6,7 @@ import ctypes as C
 import os
 import re
 import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -205,22 +206,34 @@ int main() {
                            "-I" + os.path.join(ROOT, "tests", "eigen_stub"), "-c", str(src), "-o", str(tmp_path / "eig.o")])
 
 
+_PLUGIN_PROBE = """
+import os, sys
+sys.path.insert(0, %(root)r)
+import ik_b200 as ik
+from ik_b200 import _capi as capi
+from ik_b200 import specialise as SP
+
+m = ik.Model.builtin("ur5", free_flyer=False)
+pb = ik.InverseKinematicsProblem(m, 0)
+pb.add_frame_task("tool", ik.FrameTask(m, "tool0", ik.KinematicType.Full))
+assert pb.specialisation() is None
+so = SP.build_plugin(pb, "ur5_pose_plugin")
+assert os.path.exists(so) and SP.build_plugin(pb, "ur5_pose_plugin") == so      # cached by content hash
+SP.load_plugin(so)
+SP.load_plugin(so)                                                             # idempotent
+assert pb.specialisation() == "ur5_pose_plugin"
+other = ik.InverseKinematicsProblem(m, 0)
+other.add_frame_task("tool", ik.FrameTask(m, "tool0", ik.KinematicType.Position))
+assert other.specialisation() is None
+assert capi.lib.ikb_load_specialisation(b"/nonexistent/plugin.so") == capi.ERR_INVALID_ARG
+print("REGISTERED")
+"""
+
+
 def test_plugin_specialisation_builds_and_registers():
     """ik_b200.specialise (host side, no GPU needed: nvcc cross-compiles): generator -> nvcc -> plugin .so ->
     ikb_load_specialisation; the host-only query then names the plugin for a problem built from the same URDF, and a
-    problem with another task list still has none."""
-    from ik_b200 import specialise as SP
-
-    m = ik.Model.builtin("ur5", free_flyer=False)
-    pb = ik.InverseKinematicsProblem(m, 0)
-    pb.add_frame_task("tool", ik.FrameTask(m, "tool0", ik.KinematicType.Full))
-    assert pb.specialisation() is None
-    so = SP.build_plugin(pb, "ur5_pose_plugin")
-    assert os.path.exists(so) and SP.build_plugin(pb, "ur5_pose_plugin") == so      # cached by content hash
-    SP.load_plugin(so)
-    SP.load_plugin(so)                                                             # idempotent
-    assert pb.specialisation() == "ur5_pose_plugin"
-    other = ik.InverseKinematicsProblem(m, 0)
-    other.add_frame_task("tool", ik.FrameTask(m, "tool0", ik.KinematicType.Position))
-    assert other.specialisation() is None
-    assert capi.lib.ikb_load_specialisation(b"/nonexistent/plugin.so") == capi.ERR_INVALID_ARG
+    problem with another task list still has none.  A loaded plugin stays registered until its process exits, so this
+    runs in a process of its own: other tests build the same UR5 problem and expect the table-driven kernel for it."""
+    r = subprocess.run([sys.executable, "-c", _PLUGIN_PROBE % {"root": ROOT}], capture_output=True, text=True, cwd=ROOT)
+    assert r.returncode == 0 and "REGISTERED" in r.stdout, r.stdout + r.stderr
