@@ -221,6 +221,8 @@ class pik_parameters:  # pik.hpp:13-18 + pik_data::lambda (pik.hpp:31)
         self.step_length = step_length
         self.max_time = max_time
         self.lambdas = list(lambdas) if lambdas is not None else []   # per priority level; missing levels: 1.0
+        if len(self.lambdas) > 7:
+            raise ValueError("ik::pik holds at most 7 priority levels (ikb_pik_params::lambda); got %d lambdas" % len(self.lambdas))
         self.tolerance = tolerance
 
     def c(self):
@@ -229,7 +231,7 @@ class pik_parameters:  # pik.hpp:13-18 + pik_data::lambda (pik.hpp:31)
         p.max_iterations = int(self.max_iterations)
         p.step_length = float(self.step_length)
         p.tolerance = float(self.tolerance)
-        for i, v in enumerate(self.lambdas[:7]):
+        for i, v in enumerate(self.lambdas):
             p.lam[i] = float(v)
         return p
 

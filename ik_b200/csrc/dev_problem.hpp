@@ -17,6 +17,7 @@ constexpr int kMaxFrames = 32;  // frames referenced by tasks (task frames + ref
 constexpr int kMaxRows = 48;
 constexpr int kMaxConstraints = 4;   // FrameConstraints
 constexpr int kMaxConstraintRows = 12;
+constexpr int kPikMaxLevels = 7;     // priority levels ik::pik walks (level_rows, pik_lambda2, ikb_pik_params::lambda)
 
 // Index tables of the team-per-problem kernel (dls_coop.cuh), built by build_coop_tables (problem_fill.hpp).
 constexpr int kCoopMaxPaths = 16;
@@ -54,8 +55,11 @@ template <typename T> struct alignas(16) DevProblem {
     // FrameConstraints (frame.hpp:333-465): frame / reference frame (indices into f_parent / f_placement) and KinematicType
     int32_t nconstraints, crows;
     int32_t c_frame[kMaxConstraints], c_ref[kMaxConstraints], c_type[kMaxConstraints], c_pad_[2];
-    int32_t nlevels;           // priority levels (max_priority_level + 1)
-    int32_t level_rows[7];     // rows of priority level l (stacked order = level by level); ik::pik walks them
+    // priority levels up to the highest one a task uses (not max_priority_level + 1: empty top levels cost nothing and
+    // may exceed the table).  ik::pik walks level_rows[0 .. nlevels); its entry points refuse nlevels > kPikMaxLevels,
+    // ik::dls never reads either field.
+    int32_t nlevels;
+    int32_t level_rows[kPikMaxLevels];   // rows of priority level l (stacked order = level by level)
     int32_t pad_[4];           // keeps sizeof a multiple of 16 for the bulk copy
     // Sparsity of the stacked task Jacobian, known when the problem is finalized (a frame task only touches the columns of
     // the joints between the root and its frame; SURVEY 8a: the reference's dense products ignore 60 % zeros): bit c of
@@ -101,7 +105,7 @@ template <typename T> struct SolveArgs {
     unsigned long long *list_count;   // number of entries in `list` (zeroed before the BULK launch)
     int *iters_ws;                    // step counts of suspended problems (the caller's `iters` or scratch)
     // ik::pik (generic kernel only): squared damping of every priority level (pik_data::lambda, pik.hpp:31)
-    T pik_lambda2[7];
+    T pik_lambda2[kPikMaxLevels];
     // ikb_dls_solve_ex / ikb_pik_solve_ex (team-per-problem kernel only): dls_data::dq [B][nv], stacked e [B][rows] and
     // J [B][rows][nv] of the last evaluation (data.hpp:15-28); NULL = not wanted
     T *aux_dq, *aux_e, *aux_J;

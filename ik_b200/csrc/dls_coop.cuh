@@ -444,6 +444,12 @@ IKB_HD void coop_gram_solve(const Ctx &cx, const T (*Jm)[LDM], const uint64_t *c
     for (int rr = 0; rr < RPL; ++rr) y_out[rr] = rhs[rr] * yinv[rr];
 }
 
+// Trip count of a loop whose body holds warp collectives (shfl, sync) and whose natural count `n` is per-problem data: the
+// largest `n` of the warp.  Teams of 8 or 16 lanes share a warp, and the full-mask collectives pair up the instructions of
+// all its lanes: a team that issued fewer of them than its neighbour (a level of lower rank, a team without a problem on its
+// placeholder state) would leave the neighbour waiting for good.  Trips beyond a team's own `n` do no work.
+template <class Ctx> IKB_HD int coop_warp_rounds(const Ctx &cx, int n) { return cx.warp_max(n); }
+
 // Orthonormal basis (rows of Wout, returned count = rank) of the row space of the numerically rank-r part of the mi x nv
 // matrix A (column-major with stride LD, destroyed): what A.completeOrthogonalDecomposition().pseudoInverse() * A projects
 // onto (pik.cpp:59-61, dls.cpp:44-49).  Householder QR with column pivoting, lane <-> column; rank from Eigen's threshold
@@ -473,23 +479,22 @@ IKB_HD int coop_rowspace_basis(const Ctx &cx, T (*A)[Cfg::LDX], int mi, int nv, 
             if (obn > bn || (obn == bn && obest < best)) { bn = obn; best = obest; }
         }
         if (best != k) { const unsigned char t = perm[k]; perm[k] = perm[best]; perm[best] = t; }
+        // Every branch below is data-dependent; the warp collectives are not (see coop_warp_rounds): 3 syncs per column.
         const T nrm = sqrt_(max_(bn, T(0)));
-        if (!(nrm > T(0))) {
-            if (lane == 0) diag[k] = T(0);
-            cx.sync();
-            continue;
-        }
+        const bool live = nrm > T(0);   // false for a zero (or NaN) remainder: pivot 0
         T *ck = A[perm[k]];
         const T akk = ck[k];
         const T alpha = akk >= T(0) ? -nrm : nrm;
         // v = column k below the diagonal, v[k] -= alpha; |v|^2 = 2 nrm (nrm + |akk|) (exactly what the serial sum gives up to rounding)
         T vn = T(0);
-        for (int r = k; r < mi; ++r) {
-            const T v = ck[r] - (r == k ? alpha : T(0));
-            vn += v * v;
-        }
+        if (live)
+            for (int r = k; r < mi; ++r) {
+                const T v = ck[r] - (r == k ? alpha : T(0));
+                vn += v * v;
+            }
         cx.sync();   // everybody has read column k before its owner overwrites it
-        if (vn > T(0)) {
+        const bool reflect = live && vn > T(0);
+        if (reflect) {
             const T two_over = T(2) / vn;
             for (int c = k + 1 + lane; c < nv; c += TEAM) {
                 T *col = A[perm[c]];
@@ -498,14 +503,16 @@ IKB_HD int coop_rowspace_basis(const Ctx &cx, T (*A)[Cfg::LDX], int mi, int nv, 
                 s *= two_over;
                 for (int r = k; r < mi; ++r) col[r] -= s * (ck[r] - (r == k ? alpha : T(0)));
             }
-            cx.sync();
-            if (lane == 0) {   // column k itself becomes (alpha, 0, ..., 0)
+        }
+        cx.sync();
+        if (lane == 0) {
+            if (reflect) {   // column k itself becomes (alpha, 0, ..., 0)
                 ck[k] = alpha;
                 for (int r = k + 1; r < mi; ++r) ck[r] = T(0);
             }
+            diag[k] = live ? abs_(alpha) : T(0);
         }
-        if (lane == 0) diag[k] = abs_(alpha);
-        maxpiv = max_(maxpiv, abs_(alpha));
+        if (live) maxpiv = max_(maxpiv, abs_(alpha));
         cx.sync();
     }
     const T eps = sizeof(T) == 8 ? T(2.220446049250313e-16) : T(1.1920929e-7);
@@ -521,31 +528,38 @@ IKB_HD int coop_rowspace_basis(const Ctx &cx, T (*A)[Cfg::LDX], int mi, int nv, 
     // across lanes) and the update by lane <-> column; one butterfly per row (its norm) instead of one per PAIR of rows and
     // pass -- the modified Gram-Schmidt that stood here spent a third of an ik::pik iteration in shuffles
     // (profiles/r2_s3_pik_lines.txt).  `diag` is free once the rank is known and carries the coefficients.
-    for (int r = 0; r < rank; ++r) {
+    const int rounds = coop_warp_rounds(cx, rank);
+    for (int r = 0; r < rounds; ++r) {
+        const bool live = r < rank;
         for (int pass = 0; pass < 2 && r > 0; ++pass) {
-            for (int p2 = lane; p2 < r; p2 += TEAM) {
-                T s0 = T(0), s1 = T(0);
-                int c = 0;
-                for (; c + 1 < nv; c += 2) {
-                    s0 += Wout[r][c] * Wout[p2][c];
-                    s1 += Wout[r][c + 1] * Wout[p2][c + 1];
+            if (live)
+                for (int p2 = lane; p2 < r; p2 += TEAM) {
+                    T s0 = T(0), s1 = T(0);
+                    int c = 0;
+                    for (; c + 1 < nv; c += 2) {
+                        s0 += Wout[r][c] * Wout[p2][c];
+                        s1 += Wout[r][c + 1] * Wout[p2][c + 1];
+                    }
+                    if (c < nv) s0 += Wout[r][c] * Wout[p2][c];
+                    diag[p2] = s0 + s1;
                 }
-                if (c < nv) s0 += Wout[r][c] * Wout[p2][c];
-                diag[p2] = s0 + s1;
-            }
             cx.sync();
-            for (int c = lane; c < nv; c += TEAM) {
-                T w = Wout[r][c];
-                for (int p2 = 0; p2 < r; ++p2) w -= diag[p2] * Wout[p2][c];
-                Wout[r][c] = w;
-            }
+            if (live)
+                for (int c = lane; c < nv; c += TEAM) {
+                    T w = Wout[r][c];
+                    for (int p2 = 0; p2 < r; ++p2) w -= diag[p2] * Wout[p2][c];
+                    Wout[r][c] = w;
+                }
             cx.sync();
         }
         T nr = T(0);
-        for (int c = lane; c < nv; c += TEAM) nr += Wout[r][c] * Wout[r][c];
+        if (live)
+            for (int c = lane; c < nv; c += TEAM) nr += Wout[r][c] * Wout[r][c];
         for (int off = TEAM / 2; off >= 1; off >>= 1) nr += cx.shfl(nr, lane ^ off);
-        const T inr = T(1) / sqrt_(nr);
-        for (int c = lane; c < nv; c += TEAM) Wout[r][c] *= inr;
+        if (live) {
+            const T inr = T(1) / sqrt_(nr);
+            for (int c = lane; c < nv; c += TEAM) Wout[r][c] *= inr;
+        }
         cx.sync();
     }
     cx.sync();
@@ -611,11 +625,15 @@ template <typename T, class Cfg, class Ctx>
 IKB_HD void coop_project_out(const Ctx &cx, const T (*W)[Cfg::NV], int rank, int nv, T *dq) {
     constexpr int TEAM = Cfg::TEAM;
     const int lane = cx.lane;
-    for (int r = 0; r < rank; ++r) {
+    const int rounds = coop_warp_rounds(cx, rank);
+    for (int r = 0; r < rounds; ++r) {
+        const bool live = r < rank;
         T s = T(0);
-        for (int c = lane; c < nv; c += TEAM) s += W[r][c] * dq[c];
+        if (live)
+            for (int c = lane; c < nv; c += TEAM) s += W[r][c] * dq[c];
         for (int off = TEAM / 2; off >= 1; off >>= 1) s += cx.shfl(s, lane ^ off);
-        for (int c = lane; c < nv; c += TEAM) dq[c] -= s * W[r][c];
+        if (live)
+            for (int c = lane; c < nv; c += TEAM) dq[c] -= s * W[r][c];
     }
     cx.sync();
 }
@@ -751,6 +769,7 @@ template <typename T, class Cfg, int EXTRA, class Ctx> IKB_HD void coop_init_scr
 template <int TEAM> struct CoopDevCtx {
     int lane;
     __device__ __forceinline__ void sync() const { __syncwarp(); }
+    __device__ __forceinline__ int warp_max(int v) const { return __reduce_max_sync(0xffffffffu, v); }
     __device__ __forceinline__ double shfl(double v, int src) const { return __shfl_sync(0xffffffffu, v, src, TEAM); }
     __device__ __forceinline__ float shfl(float v, int src) const { return __shfl_sync(0xffffffffu, v, src, TEAM); }
 };

@@ -162,7 +162,7 @@ static int launch_solve_impl(const ikb_problem *p, const ikb_dls_params *prm, in
     a.list = nullptr;
     a.list_count = nullptr;
     a.iters_ws = merged ? nullptr : io->iters;
-    for (int l = 0; l < 7; ++l) a.pik_lambda2[l] = pik_lambda ? (T)(pik_lambda[l] * pik_lambda[l]) : T(0);
+    for (int l = 0; l < kPikMaxLevels; ++l) a.pik_lambda2[l] = pik_lambda ? (T)(pik_lambda[l] * pik_lambda[l]) : T(0);
     if (p->spec && !pik_lambda && !aux) {
         const SpecHostConsts hc{p->hp.model.lower.data(), p->hp.model.upper.data(), p->weight_stacked.data(), p->mask_stacked.data()};
         // Scheduling (DESIGN.md 4.1).  A batch that the latency configuration keeps resident in one wave runs there
@@ -598,7 +598,10 @@ void ikb_pik_params_default(ikb_pik_params *p) {
 
 static int pik_to_dls(const ikb_problem *p, const ikb_pik_params *prm, ikb_dls_params *out) {
     if (!p || !prm) return fail(IKB_ERR_INVALID_ARG, "null argument");
-    if (p->hp.max_priority_level + 1 > 7) return fail(IKB_ERR_UNSUPPORTED, "ik::pik supports at most 7 priority levels");
+    // the kernels hold kPikMaxLevels levels (DevProblem::level_rows, SolveArgs::pik_lambda2); max_priority_level itself
+    // may be larger as long as no task sits above the table
+    if (p->hp.levels() > kPikMaxLevels)
+        return fail(IKB_ERR_UNSUPPORTED, "ik::pik holds at most 7 priority levels (ikb_pik_params::lambda): a task has priority above 6");
     ikb_dls_params_default(out);
     out->max_iterations = prm->max_iterations;
     out->step_length = prm->step_length;

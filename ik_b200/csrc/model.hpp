@@ -79,6 +79,12 @@ struct HostProblem {
         return n;
     }
 
+    int levels() const {  // one more than the highest priority any task uses
+        int n = 0;
+        for (const auto &t : tasks) n = t.priority + 1 > n ? t.priority + 1 : n;
+        return n;
+    }
+
     int rows() const;
     int e_size(int priority) const;
     int target_size() const;

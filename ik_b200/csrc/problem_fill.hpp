@@ -124,8 +124,8 @@ inline void fill_dev_problem(const HostProblem &hp, const std::vector<int> &orde
         P.c_ref[k] = lf(hp.constraints[k].ref);
         P.c_type[k] = hp.constraints[k].type;
     }
-    P.nlevels = hp.max_priority_level + 1;
-    for (int l = 0; l < 7; ++l) P.level_rows[l] = l < P.nlevels ? hp.e_size(l) : 0;
+    P.nlevels = hp.levels();
+    for (int l = 0; l < kPikMaxLevels; ++l) P.level_rows[l] = l < P.nlevels ? hp.e_size(l) : 0;
     P.tsz = hp.target_size();
     for (int j = 0; j < m.njoints(); ++j) {
         P.parent[j] = m.parent[j];

@@ -224,12 +224,15 @@ int ikb_dls_solve_ex(ikb_problem *p, const ikb_dls_params *params, const double 
  * Per iteration: dq = 0, P = I; for every priority level i: de = e_i - J_i dq, Jb = J_i P,
  * dq -= damp_pseudoinverse(Jb, lambda_i) de, P -= Jb.completeOrthogonalDecomposition().pseudoInverse() Jb; then the
  * stop test, integrate and clamp of ik::dls.  (pik_data::da, the null-space bias, is zero in the reference and not
- * exposed.)  Runs on the table-driven kernel for any tree / task mix; at most 7 priority levels. */
+ * exposed.)  Runs on the table-driven kernel for any tree / task mix. */
 typedef struct {
     int32_t max_iterations; /* 100 (pik.hpp:14) */
     double step_length;     /* 1.0 (pik.hpp:16) */
     double tolerance;       /* 1e-4 (visitor.hpp:19) */
-    double lambda[7];       /* pik_data::lambda, damping of every priority level: 1.0 (pik.hpp:31) */
+    /* pik_data::lambda, damping of every priority level: 1.0 (pik.hpp:31).  ik::pik holds at most 7 priority levels:
+     * the pik entry points return IKB_ERR_UNSUPPORTED when a task has priority 7 or more (max_priority_level itself
+     * may be larger; empty levels above the highest used one cost nothing).  ik::dls takes any priority. */
+    double lambda[7];
 } ikb_pik_params;
 void ikb_pik_params_default(ikb_pik_params *p);
 /* as ikb_dls_solve_batch / ikb_dls_solve_batch_host */

@@ -912,8 +912,16 @@ int iko_rowspace_projector(int m, int n, const double *M, double *proj) {
     return rank;
 }
 
+/* 1 when every task's priority has a lambda (below IKO_MAX_LEVELS) */
+static int pik_levels_ok(const iko_problem *pb) {
+    for (int t = 0; t < pb->ntasks; ++t)
+        if (pb->priority[t] < 0 || pb->priority[t] >= IKO_MAX_LEVELS) return 0;
+    return 1;
+}
+
 int iko_pik(const iko_model *m, const iko_problem *pb, const iko_pik_params *prm, const double *q0, const double *targets,
             double *q_out, int *iters, double *resid, double *dq_out) {
+    if (!pik_levels_ok(pb)) return -1;
     const int nq = m->nq, nv = m->nv, rows = iko_total_rows(pb), r0 = iko_e_size(pb, 0);
     double *q = (double *)malloc(sizeof(double) * nq), *qn = (double *)malloc(sizeof(double) * nq);
     double *e = (double *)malloc(sizeof(double) * (rows + 1)), *J = (double *)malloc(sizeof(double) * (rows * nv + 1));
@@ -993,8 +1001,9 @@ static void *pik_worker(void *arg) {
     return 0;
 }
 
-void iko_pik_batch(const iko_model *m, const iko_problem *pb, const iko_pik_params *prm, int B, const double *q0,
-                   const double *targets, double *q_out, unsigned char *success, int *iters, double *resid, int nthreads) {
+int iko_pik_batch(const iko_model *m, const iko_problem *pb, const iko_pik_params *prm, int B, const double *q0,
+                  const double *targets, double *q_out, unsigned char *success, int *iters, double *resid, int nthreads) {
+    if (!pik_levels_ok(pb)) return -1;
     if (nthreads < 1) nthreads = 1;
     if (nthreads > B) nthreads = B > 0 ? B : 1;
     pthread_t *th = (pthread_t *)malloc(sizeof(pthread_t) * nthreads);
@@ -1009,4 +1018,5 @@ void iko_pik_batch(const iko_model *m, const iko_problem *pb, const iko_pik_para
     if (nthreads > 1)
         for (int t = 0; t < nthreads; ++t) pthread_join(th[t], 0);
     free(th); free(jobs);
+    return 0;
 }

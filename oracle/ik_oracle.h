@@ -167,11 +167,13 @@ typedef struct {
 void iko_damp_pseudoinverse(int m, int n, const double *M, double lambda, double *out);
 /* M.completeOrthogonalDecomposition().pseudoInverse() * M (pik.cpp:59-61) -> proj n x n; returns the numerical rank */
 int iko_rowspace_projector(int m, int n, const double *M, double *proj);
+/* ik::pik on one problem / a batch.  Both return -1 and touch no output when a task's priority has no lambda (at or
+ * above IKO_MAX_LEVELS); otherwise iko_pik returns success (1/0) and iko_pik_batch 0. */
 int iko_pik(const iko_model *m, const iko_problem *pb, const iko_pik_params *prm, const double *q0,
             const double *targets, double *q_out, int *iters, double *resid, double *dq_out);
-void iko_pik_batch(const iko_model *m, const iko_problem *pb, const iko_pik_params *prm, int B, const double *q0,
-                   const double *targets, double *q_out, unsigned char *success, int *iters, double *resid,
-                   int nthreads);
+int iko_pik_batch(const iko_model *m, const iko_problem *pb, const iko_pik_params *prm, int B, const double *q0,
+                  const double *targets, double *q_out, unsigned char *success, int *iters, double *resid,
+                  int nthreads);
 
 #ifdef __cplusplus
 }

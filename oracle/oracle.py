@@ -282,6 +282,9 @@ def dls_batch(problem, q0, targets, prm=None, nthreads=1, fma=False):
     return q, ok.astype(bool), it, res
 
 
+_PIK_LEVELS = "the ik::pik oracle holds IKO_MAX_LEVELS = 8 priority levels: a task has priority 8 or more"
+
+
 class _CPikParams(C.Structure):
     _fields_ = [("max_iterations", C.c_int), ("step_length", C.c_double), ("tolerance", C.c_double),
                 ("lam", C.c_double * 8)]
@@ -315,10 +318,9 @@ def lib_f32():
     return _LIB32
 
 
-def dls_batch_f32(problem, q0, targets, prm=None, nthreads=1):
-    """ik::dls looped over a batch with number_t = float: every scalar of the restatement (model constants, FK, log6,
-    Gram, pivoted LDL^T, integrate, stop test) is single precision.  Returns float64 copies of q / resid."""
-    prm = prm or params()
+def _f32_structs(problem):
+    """The model / problem structs of `problem` with every float64 array converted to float32 (returns the structs and the
+    arrays they point into, which the caller keeps alive)."""
     m = problem.model
     keep = []
 
@@ -338,8 +340,12 @@ def dls_batch_f32(problem, q0, targets, prm=None, nthreads=1):
         return cls(*vals)
 
     pc = problem.c  # materialises problem._keep
-    cm, cp = conv(m.c, _CModelF), conv(pc, _CProblemF)
-    cprm = _CParamsF(prm.max_iterations, prm.step_length, prm.damping, prm.tolerance)
+    return conv(m.c, _CModelF), conv(pc, _CProblemF), keep
+
+
+def _f32_batch(fn, problem, q0, targets, cprm, nthreads):
+    cm, cp, keep = _f32_structs(problem)
+    m = problem.model
     q0 = np.ascontiguousarray(q0, dtype=np.float32)
     targets = np.ascontiguousarray(targets, dtype=np.float32)
     B = q0.shape[0]
@@ -348,16 +354,42 @@ def dls_batch_f32(problem, q0, targets, prm=None, nthreads=1):
     ok = np.zeros(B, dtype=np.uint8)
     it = np.zeros(B, dtype=np.int32)
     res = np.zeros(B, dtype=np.float32)
-    lib_f32().iko_dls_batch(C.byref(cm), C.byref(cp), C.byref(cprm), C.c_int(B), q0.ctypes.data_as(_fp),
-                            targets.ctypes.data_as(_fp), q.ctypes.data_as(_fp), ok.ctypes.data_as(C.POINTER(C.c_ubyte)),
-                            _pi(it), res.ctypes.data_as(_fp), C.c_int(nthreads))
-    return q.astype(np.float64), ok.astype(bool), it, res.astype(np.float64)
+    rc = getattr(lib_f32(), fn)(C.byref(cm), C.byref(cp), C.byref(cprm), C.c_int(B), q0.ctypes.data_as(_fp),
+                                targets.ctypes.data_as(_fp), q.ctypes.data_as(_fp), ok.ctypes.data_as(C.POINTER(C.c_ubyte)),
+                                _pi(it), res.ctypes.data_as(_fp), C.c_int(nthreads))
+    return rc, (q.astype(np.float64), ok.astype(bool), it, res.astype(np.float64))
+
+
+def dls_batch_f32(problem, q0, targets, prm=None, nthreads=1):
+    """ik::dls looped over a batch with number_t = float: every scalar of the restatement (model constants, FK, log6,
+    Gram, pivoted LDL^T, integrate, stop test) is single precision.  Returns float64 copies of q / resid."""
+    prm = prm or params()
+    cprm = _CParamsF(prm.max_iterations, prm.step_length, prm.damping, prm.tolerance)
+    return _f32_batch("iko_dls_batch", problem, q0, targets, cprm, nthreads)[1]
+
+
+class _CPikParamsF(C.Structure):
+    _fields_ = [("max_iterations", C.c_int), ("step_length", C.c_float), ("tolerance", C.c_float), ("lam", C.c_float * 8)]
+
+
+def pik_batch_f32(problem, q0, targets, prm=None, nthreads=1):
+    """ik::pik looped over a batch with number_t = float (the FP32 build of the same restatement: SVD damped inverse,
+    pivoted QR rank threshold with FLT_EPSILON, projector, integrate).  prm: pik_params(...).  Returns float64 copies."""
+    prm = prm or pik_params()
+    cprm = _CPikParamsF(prm.max_iterations, prm.step_length, prm.tolerance, (C.c_float * 8)(*prm.lam))
+    rc, out = _f32_batch("iko_pik_batch", problem, q0, targets, cprm, nthreads)
+    if rc != 0:
+        raise ValueError(_PIK_LEVELS)
+    return out
 
 
 def pik_params(max_iterations=100, step_length=1.0, lambdas=None, tolerance=1e-4):
     """pik.hpp:13-18 and pik_data::lambda (pik.hpp:31: 1.0 per priority level)."""
+    lambdas = list(lambdas or [])
+    if len(lambdas) > 8:
+        raise ValueError("the ik::pik oracle holds IKO_MAX_LEVELS = 8 lambdas; got %d" % len(lambdas))
     lam = (C.c_double * 8)(*([1.0] * 8))
-    for i, v in enumerate(lambdas or []):
+    for i, v in enumerate(lambdas):
         lam[i] = float(v)
     return _CPikParams(max_iterations, step_length, tolerance, lam)
 
@@ -372,6 +404,8 @@ def pik(problem, q0, targets, prm=None):
     res = C.c_double(0)
     ok = lib().iko_pik(C.byref(m.c), C.byref(problem.c), C.byref(prm), _pd(_d(q0)), _pd(_d(targets)), _pd(q),
                        C.byref(it), C.byref(res), _pd(dq))
+    if ok < 0:
+        raise ValueError(_PIK_LEVELS)
     return q, bool(ok), it.value, res.value, dq
 
 
@@ -387,8 +421,10 @@ def pik_batch(problem, q0, targets, prm=None, nthreads=1):
     ok = np.zeros(B, dtype=np.uint8)
     it = np.zeros(B, dtype=np.int32)
     res = np.zeros(B)
-    lib().iko_pik_batch(C.byref(m.c), C.byref(problem.c), C.byref(prm), C.c_int(B), _pd(q0), _pd(targets), _pd(q),
-                        ok.ctypes.data_as(C.POINTER(C.c_ubyte)), _pi(it), _pd(res), C.c_int(nthreads))
+    rc = lib().iko_pik_batch(C.byref(m.c), C.byref(problem.c), C.byref(prm), C.c_int(B), _pd(q0), _pd(targets), _pd(q),
+                             ok.ctypes.data_as(C.POINTER(C.c_ubyte)), _pi(it), _pd(res), C.c_int(nthreads))
+    if rc != 0:
+        raise ValueError(_PIK_LEVELS)
     return q, ok.astype(bool), it, res
 
 

@@ -71,6 +71,10 @@ struct HostCtx {
     double *xd;
     float *xf;
     void sync() const { team->yield(); }
+    // One team per simulated warp; `neighbour_extra` > 0 plays a neighbour team (teams of 8 / 16 lanes share a warp) whose
+    // loops run that many more trips, so the trips beyond this team's own count run too
+    int warp_max(int v) const { return v + neighbour_extra; }
+    static int neighbour_extra;
     double shfl(double v, int src) const {
         xd[lane] = v;
         team->yield();
@@ -86,6 +90,8 @@ struct HostCtx {
         return r;
     }
 };
+
+int HostCtx::neighbour_extra = 0;
 
 struct Params {
     int max_it;
@@ -147,6 +153,8 @@ void solve_cls(const HostProblem &hp, int shfl, int pik, const Params &prm, int 
 #undef RUN
 }
 }  // namespace
+
+extern "C" void coop_set_neighbour_extra(int n) { HostCtx::neighbour_extra = n; }
 
 extern "C" int coop_solve(const char *urdf, int free_flyer, int max_priority, int ntasks, const int *kind, const int *frame, const int *ref,
                           const int *type, const int *priority, const double *weights, const double *masks, int ncons,

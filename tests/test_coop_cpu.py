@@ -13,6 +13,7 @@ import pytest
 import ik_b200 as ik
 from ik_b200 import workloads as W
 from oracle import oracle as O
+from tests import pik_cases as PC
 from tests.common import make_workload, oracle_model, oracle_problem_like, urdf_text
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -225,3 +226,47 @@ def test_pik_priority_recursion(lib, lambdas):
     q, ok, it, res, _, _, _ = coop_solve(lib, pb, "cassie", True, q0, tg, O.params(max_iterations=mi), pik_lambdas=lambdas)
     assert (ok == ok_ref).all() and (it == it_ref).all()
     assert np.abs(q - q_ref).max() < 1e-7 and np.abs(res - res_ref).max() < 1e-9
+
+
+_PIK_LEVEL_CASES = {"three": (PC.cassie_three, 3), "seven": (PC.cassie_seven, 1), "empty_middle": (PC.cassie_gap, 1),
+                    "rank_deficient_middle": (PC.cassie_rank_deficient, 3), "max_priority_20": (lambda: PC.cassie_three(20), 3),
+                    "humanoid_three": (PC.humanoid_three, 2), "arm_empty_middle": (PC.arm_gap, 0)}
+
+
+@pytest.mark.parametrize("lambdas", [[1e-2, 1e-1, 1.0], []])
+@pytest.mark.parametrize("case", sorted(_PIK_LEVEL_CASES))
+def test_pik_beyond_two_levels(lib, case, lambdas):
+    """ik::pik with three to seven levels: the row-space bases of several levels stacked in the scratch and the projection
+    of J_i over all of them (J_i P, P = I - sum w w^T), an empty level between two used ones, the rank-revealing basis of
+    a rank-deficient middle level, max_priority_level 20 with tasks on levels 0-2 (the level table holds 7), and every
+    size class of the kernel (TEAM = 8, 16, 32 on the Cassie and the 32-joint tree tables).  [] = default lambdas 1.0."""
+    make, cls = _PIK_LEVEL_CASES[case]
+    c = make()
+    _, opb = c.oracle()
+    B = 6
+    mi, tol = c.stop(40)
+    q0, tg = c.workload(B, seed=23)
+    q_ref, ok_ref, it_ref, res_ref = O.pik_batch(opb, q0, tg, O.pik_params(mi, 1.0, lambdas, tol))
+    q, ok, it, res, _, _, c_cls = coop_solve(lib, c.pb, c.urdf, c.free_flyer, q0, tg, O.params(max_iterations=mi, tolerance=tol),
+                                             pik_lambdas=lambdas)
+    assert c_cls == cls
+    assert (ok == ok_ref).all() and (it == it_ref).all()
+    assert np.abs(q - q_ref).max() < 1e-7 and np.abs(res - res_ref).max() < 1e-9
+
+
+@pytest.mark.parametrize("case", ["three", "seven", "rank_deficient_middle"])
+def test_pik_warp_neighbour_with_more_rounds_changes_nothing(lib, case):
+    """Teams of 8 or 16 lanes share a warp, so the loops of the row-space basis and the projection run as many trips as
+    the largest rank in the warp (coop_warp_rounds): a neighbour's level of higher rank, or a team without a problem, must
+    not stall or change this team.  The harness plays such a neighbour (three more trips in every such loop); the results
+    are bit for bit those of a lone team."""
+    c = _PIK_LEVEL_CASES[case][0]()
+    q0, tg = c.workload(4, seed=29)
+    runs = []
+    for extra in (0, 3):
+        lib.coop_set_neighbour_extra(C.c_int(extra))
+        try:
+            runs.append(coop_solve(lib, c.pb, c.urdf, c.free_flyer, q0, tg, O.params(max_iterations=20), pik_lambdas=[1e-2, 1e-1, 1.0]))
+        finally:
+            lib.coop_set_neighbour_extra(C.c_int(0))
+    assert all(np.array_equal(a, b) for a, b in zip(runs[0][:4], runs[1][:4]))

@@ -2,9 +2,11 @@
 and row-space projector against numpy's SVD / pinv, the priority structure (a lower level never disturbs a higher one),
 and agreement with ik::dls where the two solvers coincide.  The reference itself pins nothing (no tests, cannot be built)."""
 import numpy as np
+import pytest
 
 from ik_b200 import workloads as W
 from oracle import oracle as O
+from tests import pik_cases as PC
 from tests.common import make_workload, oracle_model, oracle_problem_like
 
 RNG = np.random.default_rng(11)
@@ -84,3 +86,58 @@ def test_pik_equals_dls_on_a_single_level():
     same = okd & okp & (itd == itp) & (itd < 30)
     assert (okd == okp).mean() > 0.95 and same.mean() > 0.8
     assert np.abs(qd[same] - qp[same]).max() < 1e-7
+
+
+_LEVEL_CASES = {"three": PC.cassie_three, "seven": PC.cassie_seven, "empty_middle": PC.cassie_gap,
+                "rank_deficient_middle": PC.cassie_rank_deficient}
+
+
+@pytest.mark.parametrize("lambdas", [[1e-2, 1e-1, 1.0, 0.3, 1e-2, 0.5, 1e-1], []])
+@pytest.mark.parametrize("case", sorted(_LEVEL_CASES))
+def test_pik_step_matches_numpy_beyond_two_levels(case, lambdas):
+    """The oracle's step for N levels against numpy's SVD / pinv rebuild of pik.cpp:44-62, including an empty level between
+    two used ones and a level whose J_i P loses rank; then the priority property: what levels below k add to dq leaves
+    J_k's task velocity alone, J_k (dq - dq_after_k) = 0, for every level that keeps its rank."""
+    c = _LEVEL_CASES[case]()
+    _, opb = c.oracle()
+    lam = [1.0] * 7 if not lambdas else lambdas
+    q0, tg = c.workload(12, seed=19)
+    for b in range(12):
+        e, J = opb.evaluate(q0[b], tg[b])
+        dq, after = PC.numpy_pik_step(e, J, c.levels, lam)
+        _, _, _, _, dq_o = O.pik(opb, q0[b], tg[b], O.pik_params(max_iterations=1, lambdas=lambdas))
+        assert np.abs(dq_o - dq).max() < 1e-9
+        row = 0
+        for k, mi in enumerate(c.levels):
+            if mi and k not in c.deficient:
+                assert np.abs(J[row:row + mi] @ (dq - after[k])).max() < 1e-9
+            row += mi
+        if c.deficient:   # the level really loses rank after the projection: one direction, far below the others
+            k = min(c.deficient)
+            r0 = sum(c.levels[:k])
+            Jk = J[r0:r0 + c.levels[k]]
+            P = np.eye(J.shape[1]) - np.linalg.pinv(J[:r0]) @ J[:r0]
+            s = np.linalg.svd(Jk @ P, compute_uv=False)
+            assert s[-2] > 1e-3 and s[-1] < 1e-12
+
+
+def test_pik_oracle_level_capacity():
+    """IKO_MAX_LEVELS (8) lambdas at most; a task on level 8 is refused instead of reading past the lambda table, while
+    levels declared but unused above the last task cost nothing."""
+    with pytest.raises(ValueError):
+        O.pik_params(lambdas=[1.0] * 9)
+    c = PC.cassie_three(max_priority_level=20)
+    _, opb = c.oracle()
+    _, opb3 = PC.cassie_three().oracle()
+    q0, tg = c.workload(4, seed=5)
+    a, b = O.pik_batch(opb, q0, tg), O.pik_batch(opb3, q0, tg)
+    assert all(np.array_equal(x, y) for x, y in zip(a, b))
+    om = oracle_model("cassie")
+    opb = O.Problem(om, 8)
+    opb.add_frame_task("LeftFootFront", O.POSITION, priority=8)
+    with pytest.raises(ValueError):
+        O.pik_batch(opb, q0[:1], tg[:1, :12])
+    with pytest.raises(ValueError):
+        O.pik(opb, q0[0], tg[0, :12])
+    with pytest.raises(ValueError):
+        O.pik_batch_f32(opb, q0[:1], tg[:1, :12])
