@@ -11,7 +11,7 @@ CSRC := ik_b200/csrc
 OBJ := build/obj
 LIB := ik_b200/libikb200.so
 GEN := $(CSRC)/gen
-SPECS := cassie_feet_pelvis cassie_feet_pelvis_arrow cassie_feet_pelvis_arrow_b cassie_feet_pelvis_w1 cassie_feet_pelvis_w2 manipulator_tool humanoid_limbs humanoid_limbs_arrow cassie_demo cassie_demo_posture
+SPECS := cassie_feet_pelvis cassie_feet_pelvis_arrow cassie_feet_pelvis_fold cassie_feet_pelvis_arrow_b cassie_feet_pelvis_w1 cassie_feet_pelvis_w2 manipulator_tool humanoid_limbs humanoid_limbs_arrow cassie_demo cassie_demo_posture
 GEN_HDRS := $(patsubst %,$(GEN)/%.cuh,$(SPECS))
 
 SRCS_CU := $(wildcard $(CSRC)/*.cu)

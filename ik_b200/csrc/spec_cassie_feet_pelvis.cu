@@ -4,7 +4,8 @@
 // BULK (throughput): thread-per-problem, generated arithmetic; three decompositions are compiled
 // (ik_b200/specs/cassie_feet_pelvis*.json): one warp role (W1), two (pelvis+left | right+solve, W2) and three
 // (pelvis+solve | left | right, W3, with presolve); W3 is the measured-best one for both scalar types, IKB_CASSIE_ROLES=1|2|3
-// overrides it (tools/bench_variants.sh).
+// overrides it (tools/bench_variants.sh).  The merged FP64 BULK launch of W3 runs the arrow step with the pelvis folded into
+// the two leg roles (cassie_feet_pelvis_fold: 6 groups = 192 problems per SM, Jacobian rows in tensor memory).
 // TAIL (latency): the team-per-problem kernel of dls_team.cuh -- 16 lanes share one problem -- for the stragglers a BULK
 // launch suspends and for batches too small to fill the GPU.  IKB_CASSIE_TAIL=0 selects the previous latency
 // configuration (W3, one 32-problem group per CTA) for A/B measurements.
@@ -16,6 +17,7 @@
 #include "gen/cassie_feet_pelvis.cuh"
 #include "gen/cassie_feet_pelvis_arrow.cuh"
 #include "gen/cassie_feet_pelvis_arrow_b.cuh"
+#include "gen/cassie_feet_pelvis_fold.cuh"
 #include "gen/cassie_feet_pelvis_w1.cuh"
 #include "gen/cassie_feet_pelvis_w2.cuh"
 
@@ -26,16 +28,20 @@ using SA = SpecCassieFeetPelvisArrow;  // three roles, bordered-block-diagonal s
 using S2 = SpecCassieFeetPelvisW2;
 using S1 = SpecCassieFeetPelvisW1;
 using SB = SpecCassieFeetPelvisArrowB;  // ... factor / y in registers, free-flyer stepped once by the pelvis role
-// IKB_CASSIE_SOLVE=dense|arrow|arrowb (A/B runs).  (Solving the shared-column system on the pelvis role alone --
+// ... two roles (left | right leg), each evaluating the pelvis pose in registers and publishing half of its share of the
+// shared-column system: no idle pelvis warp, so 6 groups of 2 warps fit where 4 groups of 3 did (same arithmetic as SA)
+using SF = SpecCassieFeetPelvisFold;
+// IKB_CASSIE_SOLVE=dense|arrow|arrowb|fold (A/B runs).  (Solving the shared-column system on the pelvis role alone --
 // spec option arrow_cap_solo -- was measured too: 3.13 ms against 3.10 ms for 8 x 65 536, not kept.)
 int solve_variant(bool f64, bool tail) {
     const char *e = std::getenv("IKB_CASSIE_SOLVE");
     if (e && std::strcmp(e, "dense") == 0) return 0;
     if (e && std::strcmp(e, "arrow") == 0) return 1;
     if (e && std::strcmp(e, "arrowb") == 0) return 2;
-    // the throughput launch in FP64 is register-bound (168 per thread): factor in shared memory; everything else has
-    // registers to spare (the three arrow variants run the same arithmetic: bit-identical results, measured)
-    return (f64 && !tail) ? 1 : 2;
+    if (e && std::strcmp(e, "fold") == 0) return 3;
+    // the throughput launch in FP64 is register-bound (168 per thread): factor in shared memory, pelvis folded into the
+    // leg roles; everything else has registers to spare (the arrow variants run the same arithmetic: bit-identical results)
+    return (f64 && !tail) ? 3 : 2;
 }
 int roles(int dflt) {
     const char *e = std::getenv("IKB_CASSIE_ROLES");
@@ -112,6 +118,9 @@ template <typename T> int launch(const SpecHostConsts &hc, const SolveArgs<T> &a
         switch (solve_variant(sizeof(T) == 8, true)) {
             case 0: return launch_spec_tail<S3, T>(hc, a, n, sms, s);
             case 1: return launch_spec_tail<SA, T>(hc, a, n, sms, s);
+            case 3:
+                if constexpr (sizeof(T) == 8) return launch_spec_tail<SF, T>(hc, a, n, sms, s);
+                return launch_spec_tail<SB, T>(hc, a, n, sms, s);
             default: return launch_spec_tail<SB, T>(hc, a, n, sms, s);
         }
     }
@@ -120,6 +129,12 @@ template <typename T> int launch(const SpecHostConsts &hc, const SolveArgs<T> &a
             switch (solve_variant(sizeof(T) == 8, false)) {
                 case 0: return launch_spec_bulk<S3, T>(hc, a, n, sms, s);
                 case 1: return launch_spec_bulk<SA, T>(hc, a, n, sms, s);
+                case 3:   // (FP64 only: in FP32 the Jacobian rows would have to stay in shared memory)
+                    // A merged launch of the queue (several batches) runs SF: 2.40 -> 2.09 ms per launch, 203 -> 230 M
+                    // solves/s (B200).  A lone batch keeps SA: with SF its BULK + TAIL pair took 0.82 instead of 0.79 ms --
+                    // 192 slots per SM still hold more problems when the queue runs dry, and the TAIL launch gets them.
+                    if constexpr (sizeof(T) == 8) return a.nseg > 0 ? launch_spec_bulk<SF, T>(hc, a, n, sms, s) : launch_spec_bulk<SA, T>(hc, a, n, sms, s);
+                    return launch_spec_bulk<SB, T>(hc, a, n, sms, s);
                 default: return launch_spec_bulk<SB, T>(hc, a, n, sms, s);
             }
         case 2: return launch_spec_bulk<S2, T>(hc, a, n, sms, s);

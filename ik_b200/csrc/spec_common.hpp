@@ -28,6 +28,9 @@ template <typename T, int STRIDE> struct Strip {
     IKB_HD void set(int k, T v) const { base[k * STRIDE] = v; }
     IKB_HD T get(int k) const { return base[k * STRIDE]; }
     IKB_HD T operator[](int k) const { return base[k * STRIDE]; }
+    template <int N> IKB_HD void getn(int k, T (&v)[N]) const {   // (TStrip: one tensor-memory wait for the whole run)
+        for (int i = 0; i < N; ++i) v[i] = base[(k + i) * STRIDE];
+    }
     IKB_HD void flush() const {}   // (TStrip, tmem_scratch.cuh: wait for the asynchronous stores)
     // element k <- *src, asynchronously on the device (cp.async: global -> shared without a register in between, so a
     // whole pose is in flight at once and its latency is paid once); the copying thread calls strip_copies_wait() before

@@ -95,7 +95,56 @@ template <typename T> struct TStrip {
         asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
         return __hiloint2double((int)hi, (int)lo);
     }
+    // elements k .. k + N - 1 with ONE wait: power-of-two runs of columns per tcgen05.ld, then tcgen05.wait::ld (a block
+    // of generated code that reads several consecutive slots pays one tensor-memory latency instead of N)
+    template <int N> __device__ __forceinline__ void getn(int k, T (&v)[N]) const {
+        uint32_t r[2 * N];
+        tmem_ld_run<2 * N>(base + (uint32_t)(k * 2), r);
+        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+        for (int i = 0; i < 2 * N; ++i) asm volatile("" : "+r"(r[i]));   // no use of a loaded register moves above the wait
+#pragma unroll
+        for (int i = 0; i < N; ++i) v[i] = __hiloint2double((int)r[2 * i + 1], (int)r[2 * i]);
+    }
     __device__ __forceinline__ void flush() const { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
+
+  private:
+    template <int C> __device__ __forceinline__ static void ld_cols(uint32_t a, uint32_t *r) {
+        if constexpr (C == 16) {
+            asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+                         : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
+                           "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+                         : "r"(a)
+                         : "memory");
+        } else if constexpr (C == 8) {
+            asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+                         : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+                         : "r"(a)
+                         : "memory");
+        } else if constexpr (C == 4) {
+            asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"
+                         : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3])
+                         : "r"(a)
+                         : "memory");
+        } else {
+            static_assert(C == 2, "runs are cut into 16, 8, 4 and 2 columns");
+            asm volatile("tcgen05.ld.sync.aligned.32x32b.x2.b32 {%0, %1}, [%2];" : "=r"(r[0]), "=r"(r[1]) : "r"(a) : "memory");
+        }
+    }
+    template <int NC> __device__ __forceinline__ static void tmem_ld_run(uint32_t a, uint32_t *r) {
+        if constexpr (NC >= 16) {
+            ld_cols<16>(a, r);
+            tmem_ld_run<NC - 16>(a + 16, r + 16);
+        } else if constexpr (NC >= 8) {
+            ld_cols<8>(a, r);
+            tmem_ld_run<NC - 8>(a + 8, r + 8);
+        } else if constexpr (NC >= 4) {
+            ld_cols<4>(a, r);
+            tmem_ld_run<NC - 4>(a + 4, r + 4);
+        } else if constexpr (NC >= 2) {
+            ld_cols<2>(a, r);
+        }
+    }
 };
 
 // (single precision has registers to spare: never parked)

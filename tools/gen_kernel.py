@@ -28,6 +28,7 @@ revolute and prismatic joints; FrameTask (Position / Orientation / Full) with th
 Anything else runs on the generic kernel.
 """
 import json
+import re
 import sys
 
 J_UNIVERSE, J_FF, J_RX, J_RY, J_RZ, J_RU, J_PX, J_PY, J_PZ, J_PU = range(10)
@@ -209,6 +210,9 @@ class Generator:
         self.mir = None
         # role-local configuration registers (arrow specs): global q index -> index into the role's own T q[NQL]
         self.qmap = None
+        # spec "fold_task" (gen_fold): slot / row -> name of the register that holds the fold task's Jacobian entry / error
+        self.jreg = None
+        self.ereg = None
 
     def ql(self, iq):
         """register index of configuration scalar iq in the code being emitted (role-local for arrow specs)"""
@@ -464,6 +468,9 @@ class Generator:
             src = {POSITION: ["lin%d[%d]" % (n, i) for i in range(3)], ORIENTATION: ["w%d[%d]" % (n, i) for i in range(3)],
                    FULL: ["lin%d[%d]" % (n, i) for i in range(3)] + ["w%d[%d]" % (n, i) for i in range(3)]}[kt]
             for i, s in enumerate(src):
+                if self.jreg is not None:   # fold task: the weighted error stays in a register (fold_publish stores it)
+                    self.ereg[row + i] = E.var("%s * %s" % (wexpr(row + i), s), "ev")
+                    continue
                 E.raw("%s.set(%d, %s * %s);" % (sEn, row + i, wexpr(row + i), s))
             top = kt in (POSITION, FULL)
             bot = kt in (ORIENTATION, FULL)
@@ -473,6 +480,9 @@ class Generator:
 
             def store(r, col, val):
                 k = self.slot(r, col)
+                if self.jreg is not None:   # fold task: the entry never leaves the registers
+                    self.jreg[k] = E.var("%s * %s" % (wexpr(r), lit(val)), "jv")
+                    return
                 E.raw("%s.set(%d, %s * %s);  // J[%d][%d]" % (sJn, k, wexpr(r), lit(val), r, col))
 
             chain = task["chain"]
@@ -1129,7 +1139,29 @@ class Generator:
         self.rhs_off = RHS
         return grams, L
 
-    def gen_solve_arrow(self, groups, solver):
+    def tmem_batch(self, lines, strip, ind):
+        """Spec "tmem_j": the Jacobian reads of a block of generated lines become one getn() per run of consecutive slots,
+        issued at the top of the block -- a few tcgen05.ld and ONE wait per run (TStrip::getn) instead of a load and a wait
+        per entry.  The same values reach the same expressions."""
+        if not self.spec.get("tmem_j"):
+            return lines
+        pat = re.compile(r"\b%s\.get\((-?\d+)\)" % strip)
+        runs = []
+        for k in sorted({int(k) for ln in lines for k in pat.findall(ln)}):
+            if runs and runs[-1][0] + runs[-1][1] == k:
+                runs[-1][1] += 1
+            else:
+                runs.append([k, 1])
+        head, name = [], {}
+        for k0, n in runs:
+            nm = "jb%d" % k0 if k0 >= 0 else "jbm%d" % -k0
+            head.append(ind + "T %s[%d];" % (nm, n))
+            head.append(ind + "%s.getn(%d, %s);" % (strip, k0, nm))
+            for i in range(n):
+                name[k0 + i] = "%s[%d]" % (nm, i)
+        return head + [pat.sub(lambda mt: name[int(mt.group(1))], ln) for ln in lines]
+
+    def gen_solve_arrow(self, groups, solver, fold=None):
         """Spec "arrow_solve": the step WITHOUT the dense M x M factorisation, for task sets whose Jacobian is "bordered block
         diagonal": a few columns (the free-flyer; joints that several limbs' tasks share) are touched by several warp
         roles, every other column by ONE role only.  With U_a / C_a the shared / private columns of role a's rows,
@@ -1151,7 +1183,9 @@ class Generator:
         Strip layout (sL): e (M, written by evaluate, never overwritten) | s (k) | per role: published S'_a, t'_a and, for a
         role with private columns, the factor of D_a (whose slots finally carry y_a).  A role WITHOUT private columns
         publishes into its own Jacobian slots instead (nobody else reads them, and it has them in registers by then).
-        Roles of a mirrored task pair share one body (`side` rebases the strips), as their evaluate does."""
+        Roles of a mirrored task pair share one body (`side` rebases the strips), as their evaluate does.
+        `fold`: index of the group that is the spec's "fold_task" (no warp role of its own, see gen_fold): its contributions
+        are published from registers by gen_fold, in the factor strip; the warp role of group k is then k - 1."""
         M = self.rows
         R = len(groups)
         ind = "        "
@@ -1198,7 +1232,7 @@ class Generator:
         facb = {}    # role -> base of its factor (m (m + 1) / 2 slots) in sL
         for k in range(R):
             own = sorted(self.slots[(r, c)] for (r, c) in self.slots if row_role[r] == k)
-            if not privs[k] and len(own) >= per and self.spec.get("arrow_pub_in_j", True) and not self.spec.get("tmem_j"):
+            if not privs[k] and len(own) >= per and self.spec.get("arrow_pub_in_j", True) and not self.spec.get("tmem_j") and k != fold:
                 pub[k] = ("J", own[:per])
             else:
                 pub[k] = ("L", off)
@@ -1213,7 +1247,7 @@ class Generator:
         if ncq and not fac_regs:
             mail = {}
             for k in range(R):
-                if k == solver:
+                if k == solver or k == fold:
                     continue
                 m = len(role_rows[k])
                 own = ([facb[k] + i for i in range(m * (m + 1) // 2)] if privs[k] else []) + list(role_rows[k])   # (e row r sits in slot r)
@@ -1225,8 +1259,8 @@ class Generator:
                     mail = None
                     break
                 mail[k] = own[:ncq]
-            if mail is not None and not privs[solver]:
-                self.arrow_mail = mail
+            if mail is not None and (not privs[solver] or fold is not None):
+                self.arrow_mail = {k - (fold is not None): v for k, v in mail.items()}   # keyed by warp role
                 y_regs = True      # (y must not sit in the factor slots: the solver role fills the mailboxes while the others step)
         self.arrow_y = {}   # row -> sL slot of y[row] (rows of roles with private columns)
 
@@ -1284,13 +1318,15 @@ class Generator:
             for pc, c in enumerate(priv):
                 need = [i for i in range(m) if has(rows[i], c)]
                 L.append(ind + "{  // private column #%d" % pc)
+                blk = []
                 for i in need:
-                    L.append(ind + "    const T a%d = %s;" % (i, jget(rows[i], c)))
+                    blk.append(ind + "    const T a%d = %s;" % (i, jget(rows[i], c)))
                 for i in need:
                     for j in need:
                         if i >= j:
-                            L.append(ind + "    d%d_%d += a%d * a%d;" % (i, j, i, j))
+                            blk.append(ind + "    d%d_%d += a%d * a%d;" % (i, j, i, j))
                             nf[k] += 1
+                L.extend(self.tmem_batch(blk, "sJr", ind + "    "))
                 L.append(ind + "}")
             # ---- LDL^T in registers (SPD thanks to the damping: no pivoting) ----
             fi = 0
@@ -1340,6 +1376,8 @@ class Generator:
             for a_, c in enumerate(ush):
                 L.append(ind + "IKB_PHASE_FENCE();")
                 L.append(ind + "{  // shared column %d" % c)
+                L0 = L
+                L = []
                 for i in range(m):
                     if has(rows[i], c):
                         L.append(ind + "const T u%d_%d = %s;" % (i, spos[c], jget(rows[i], c)))
@@ -1355,6 +1393,7 @@ class Generator:
                 L.append(pset(KK + spos[c], "damping2 * (%s)" % (" + ".join(terms) if terms else "T(0)")))
                 entries.setdefault(("t", spos[c]), set()).add(k)
                 nf[k] += len(terms)
+                L = L0 + self.tmem_batch(L, "sJr", ind)
                 L.append(ind + "}")
             # ---- phase 3: y_a = D_a^-1 (e_a - U_a s) ----
             for i in range(m):
@@ -1366,6 +1405,7 @@ class Generator:
             for j, idx in sorted(fac_inv.items()):
                 F.append(ind + ("const T fi%d = fac[%d];" % (j, idx) if fac_regs else "const T fi%d = sLr.get(%d);" % (j, idx - dL)))
             w = solve_lines(F, ["r%d" % i for i in range(m)], "y_", lname=lambda i, j: "fl%d_%d" % (i, j), iname=lambda j: "fi%d" % j)
+            F[:] = self.tmem_batch(F, "sJr", ind)
             if y_regs:
                 for i in range(m):
                     F.append(ind + "y[%d] = %s;" % (i, w[i] if w[i] else "T(0)"))
@@ -1403,6 +1443,16 @@ class Generator:
                 mirror_of[rb] = (ra, dJ, dR, dL)
         locals_, finishes = [], []
         for k in range(R):
+            if k == fold:
+                if privs[k] or pub[k][0] != "L":
+                    raise ValueError("fold_task: its rows must touch shared columns only")
+                self.fold_pub = self.gen_fold_publish(role_rows[k], ushs[k], has, spos, KK, pub[k][1], R - 1)
+                for key in self.fold_pub[1]:
+                    entries.setdefault(key, set()).add(k)
+                nf[k] = self.fold_pub[2]
+                locals_.append([])
+                finishes.append([])
+                continue
             hdr = ind + "// role %d: rows %s, private columns %s, shared columns %s" % (k, role_rows[k], privs[k], ushs[k])
             L, F = emit_role(k)
             locals_.append([hdr] + L)
@@ -1436,6 +1486,38 @@ class Generator:
         self.rhs_off = 0
         return locals_, Cc, finishes
 
+    def gen_fold_publish(self, rows, ush, has, spos, KK, off, nw):
+        """Spec "fold_task": the contributions of the fold task's rows to the shared-column system (U^T U and U^T e -- the rows
+        have no private columns, so D = l^2 I cancels), with the SAME terms in the same order as a warp role of its own
+        publishes them (gen_solve_arrow, branch `not priv`), but straight from the registers of the fold task's evaluation,
+        which every warp role runs.  The rows are cut into nw consecutive runs, run w belonging to warp role w: the role
+        stores the weighted errors of its rows, and an entry is published by the role that owns the last row among its
+        terms (Cassie's pelvis: role 0 the 18 entries of the position rows, role 1 the 9 that also involve the orientation
+        rows -- 54 FMAs each).  Returns (lines per warp role, published entries, FMAs)."""
+        m = len(rows)
+        own = {r: i * nw // m for i, r in enumerate(rows)}
+        code = [[] for _ in range(nw)]
+        keys, nfma = [], 0
+        for r in rows:
+            code[own[r]].append("sE.set(%d, %s);" % (r, self.ereg[r]))
+
+        def u(i, c):
+            return self.jreg[self.slots[(rows[i], c)]]
+
+        for a_, c in enumerate(ush):
+            for c2 in ush[:a_ + 1]:
+                idx = [i for i in range(m) if has(rows[i], c) and has(rows[i], c2)]
+                if idx:
+                    at = off + spos[c] * (spos[c] + 1) // 2 + spos[c2]
+                    code[own[rows[idx[-1]]]].append("sE.set(%d, %s);" % (at, " + ".join("%s * %s" % (u(i, c), u(i, c2)) for i in idx)))
+                    keys.append((spos[c], spos[c2]))
+                    nfma += len(idx)
+            idx = [i for i in range(m) if has(rows[i], c)]
+            code[own[rows[idx[-1]]]].append("sE.set(%d, %s);" % (off + KK + spos[c], " + ".join("%s * %s" % (u(i, c), self.ereg[rows[i]]) for i in idx)))
+            keys.append(("t", spos[c]))
+            nfma += len(idx)
+        return code, keys, nfma
+
     def gen_step_roles_arrow(self, groups, solver):
         """step_role() of spec "arrow_solve": dq of a shared column is -s (from the strip), a private column's comes from the
         role's own rows of y; the joints common to all roles (the free-flyer) are stepped by everybody, redundantly."""
@@ -1464,7 +1546,9 @@ class Generator:
             cols, qs = self.joint_cols(own)
             self.qmap = self.qmaps[k] if self.qmaps else None
             self.ymap = {r: v[1] for r, v in self.arrow_y.items() if isinstance(v, tuple)} or None   # y in the role's registers
-            roles.append(dq_lines(cols, ind + "    ") + self.gen_integrate(own, ind + "    "))
+            # (one run per column: the whole role's block at once would hold 2 x 21 more registers across the step)
+            dq = [b for ln in dq_lines(cols, ind + "    ") for b in self.tmem_batch([ln], "sJ", ind + "    ")]
+            roles.append(dq + self.gen_integrate(own, ind + "    "))
             qsets.append(qs + (cqs if k == solver else []))
         self.qmap = None
         self.ymap = None
@@ -1547,8 +1631,15 @@ class Generator:
 
     def emit(self, struct_name, display_name):
         groups = self.spec.get("warp_groups") or [list(range(len(self.tasks)))]
-        if sorted(t for g in groups for t in g) != list(range(len(self.tasks))):
-            raise ValueError("warp_groups must partition the task list")
+        # "fold_task": a task whose rows touch only the columns shared by all roles (Cassie's pelvis pose: the free-flyer) and
+        # that has no warp role of its own -- every role evaluates it in registers and publishes its share of the task's
+        # contributions to the shared-column system (gen_fold_publish).  The solve sees it as a group of its own (`units`).
+        fold = self.spec.get("fold_task")
+        folds = [fold] if fold is not None else []
+        units = [folds] + groups if folds else groups
+        wsh = len(folds)   # group k of `units` is warp role k - wsh
+        if sorted(t for g in units for t in g) != list(range(len(self.tasks))):
+            raise ValueError("warp_groups (and fold_task) must partition the task list")
         solver = int(self.spec.get("solver_warp", 0))
         # mirrored task pairs (each alone in its warp role) share ONE evaluate body
         mirrors = {}   # role index -> (shared body id, side)
@@ -1561,6 +1652,8 @@ class Generator:
             mirrors[rb] = (len(shared), 1)
             shared.append(None)
         arrow = bool(self.spec.get("arrow_solve")) and len(groups) > 1
+        if folds and not (arrow and self.tasks[fold]["kind"] == "frame"):
+            raise ValueError("fold_task needs arrow_solve, two or more warp roles and a frame task")
         self.qmaps = None
         nql = self.nq
         if arrow and self.spec.get("local_q", True):
@@ -1568,8 +1661,10 @@ class Generator:
             # writes) -- the joints common to all roles first (same registers in every role), then its own chains; mirrored
             # roles keep corresponding joints in the same registers, so their shared body needs no select.  (With one
             # T q[NQ] for all roles every coordinate is live in every warp: 2 NQ registers in FP64.)
-            chains = [sorted(set(j for t in g for j in self.tasks[t]["chain"])) for g in groups]
+            chains = [sorted(set(j for t in g + folds for j in self.tasks[t]["chain"])) for g in groups]
             common = sorted(set.intersection(*[set(ch) for ch in chains]))
+            if folds and not set(self.tasks[fold]["chain"]) <= set(common):
+                raise ValueError("fold_task: its chain must be common to all warp roles")
             covered = set(j for ch in chains for j in ch)
             loose = [j for j, jt in enumerate(self.joints) if jt["type"] != J_UNIVERSE and j not in covered]
             self.qmaps = []
@@ -1580,6 +1675,16 @@ class Generator:
                         mp[iq] = len(mp)
                 self.qmaps.append(mp)
             nql = max(len(mp) for mp in self.qmaps)
+        fold_ev = None
+        if folds:
+            # first, so that its (never stored) Jacobian entries take the first slots and every warp role's slots follow
+            self.qmap = self.qmaps[0] if self.qmaps else None   # (its coordinates sit in the same registers in every role)
+            self.jreg, self.ereg = {}, {}
+            Ef = Emitter(prefix="f")
+            self.gen_task(Ef, fold, {})
+            fold_ev = Ef.lines
+            self.fold_regs = (self.jreg, self.ereg)
+            self.jreg = self.ereg = None
         evs = []
         for k, g in enumerate(groups):
             self.qmap = self.qmaps[k] if self.qmaps else None
@@ -1619,7 +1724,10 @@ class Generator:
         uniform = bool(self.spec.get("uniform_solve")) and bool(self.spec.get("parallel_solve")) and len(groups) > 1
         if arrow:
             uniform = False
-            arrow_code = self.gen_solve_arrow(groups, solver)
+            if folds:
+                self.jreg, self.ereg = self.fold_regs
+            arrow_code = self.gen_solve_arrow(units, solver + wsh, 0 if folds else None)
+            self.jreg = self.ereg = None
             nfact = max(self.arrow["nfact"], rows + self.nq)   # layout: see gen_solve_arrow
             self.eoff = 0
         if uniform:
@@ -1653,7 +1761,8 @@ class Generator:
         out.append("    static constexpr bool ARROW = %s;" % ("true" if arrow else "false"))
         # Jacobian slots per role (every slot belongs to the role that evaluates its row; a role's slots are consecutive)
         row_role_ = {self.tasks[t]["row"] + i: k for k, g in enumerate(groups) for t in g for i in range(self.tasks[t]["dim"])}
-        jslots = [sorted(sl for (r, c_), sl in self.slots.items() if row_role_[r] == k) for k in range(len(groups))]
+        # (the fold task's entries are never stored: they belong to no role's slots)
+        jslots = [sorted(sl for (r, c_), sl in self.slots.items() if row_role_.get(r) == k) for k in range(len(groups))]
         contiguous = all(js == list(range(js[0], js[0] + len(js))) for js in jslots if js)
         tmemj = bool(arrow and self.spec.get("tmem_j") and contiguous)
         out.append("    // TMEMJ: every role reads and writes only its own rows of J, and this spec asks the FP64 kernel to keep them in")
@@ -1689,10 +1798,13 @@ class Generator:
             out.append("    // copy this role's target poses into the strip sT")
             out.append("    template <typename T, typename S>")
             out.append("    static IKB_HD void load_targets_w%d(const T *tg, long long es, const S &sT) {" % k)
-            for t in g:
-                toff = self.tasks[t]["toff"]
+            spans = [(self.tasks[t]["toff"], self.tasks[t]["toff"] + self.tasks[t]["tsize"]) for t in g]
+            for t in folds:   # the fold task's target: its own share (every role reads all of it behind the barrier at the top of a trip)
+                t0, n = self.tasks[t]["toff"], self.tasks[t]["tsize"]
+                spans.append((t0 + k * n // len(groups), t0 + (k + 1) * n // len(groups)))
+            for a_, b_ in spans:
                 out.append("#pragma unroll")
-                out.append("        for (int k = %d; k < %d; ++k) sT.copy_in(k, tg + k * es);  // asynchronous: strip_copies_wait() before evaluate" % (toff, toff + self.tasks[t]["tsize"]))
+                out.append("        for (int k = %d; k < %d; ++k) sT.copy_in(k, tg + k * es);  // asynchronous: strip_copies_wait() before evaluate" % (a_, b_))
             out.append("    }")
             if ev is None:
                 continue
@@ -1700,6 +1812,17 @@ class Generator:
             out.append("    template <typename T, typename S>")
             out.append("    static IKB_HD void evaluate_w%d(const T (&q)[NQL], const S &tg, const SpecConsts<T, NQ, M> &c, const S &sJ, const S &sE) {" % k)
             out.extend(ev)
+            out.append("    }")
+        if folds:
+            out.append("    // ---- fold task %d (%s): every role evaluates it in registers; role k stores its share of the rows / contributions ----" %
+                       (fold, self.tasks[fold]["name"]))
+            out.append("    template <typename T, typename S>")
+            out.append("    static IKB_HD void evaluate_f(const int role, const T (&q)[NQL], const S &tg, const SpecConsts<T, NQ, M> &c, const S &sE) {")
+            out.extend(fold_ev)
+            for k, code in enumerate(self.fold_pub[0]):
+                out.append("        if (role == %d) {" % k)
+                out.extend("            " + ln for ln in code)
+                out.append("        }")
             out.append("    }")
         for bid, body in enumerate(shared):
             out.append("    // ---- shared by the roles of the mirrored tasks %s (side = 0 / 1) ----" % (self.spec["mirror"][bid],))
@@ -1715,6 +1838,8 @@ class Generator:
         out.append("    }")
         out.append("    template <typename T, typename S>")
         out.append("    static IKB_HD void evaluate(int role, const T (&q)[NQL], const S &tg, const SpecConsts<T, NQ, M> &c, const S &sJ, const S &sE) {")
+        if folds:
+            out.append("        evaluate_f(role, q, tg, c, sE);")
         for k in range(len(groups)):
             if k not in mirrors:
                 out.append("        if (role == %d) evaluate_w%d(q, tg, c, sJ, sE);" % (k, k))
@@ -1757,9 +1882,10 @@ class Generator:
             out.append("    // strip sL: e [0, %d) | s [%d, %d) | published contributions %s | factors / y %s" %
                        (rows, A["soff"], A["soff"] + A["ks"], {k: v if v[0] == "L" else "own J slots" for k, v in A["pub"].items()}, A["facb"]))
             partner = {ra: rb for rb, (ra, _, _, _) in A["mirror_of"].items()}
-            for k in range(len(groups)):
-                if k in A["mirror_of"]:
-                    continue   # runs the body of its mirror partner
+            nu, su = len(units), solver + wsh   # (groups of the solve and the SOLVER role's group; role of group k: k - wsh)
+            for k in range(nu):
+                if k in A["mirror_of"] or k < wsh:
+                    continue   # runs the body of its mirror partner / the fold task publishes from its evaluate
                 if k in partner:
                     _, dJ, dR, dL = A["mirror_of"][partner[k]]
                     sig = "const int side, "
@@ -1794,16 +1920,18 @@ class Generator:
             out.append("    template <typename T, typename S, typename SYNC, typename HOOK>")
             out.append("    static IKB_HD void psolve(int role, const S &sJ, const S &sL, const S &sE, T damping2, T (&y)[MY], SYNC &sync, HOOK &hook) {")
             out.append("        T s[%d], fac[%d];" % (A["ks"], A["nfac"]))
-            for k in range(len(groups)):
-                if k in A["mirror_of"]:
+            for k in range(nu):
+                if k in A["mirror_of"] or k < wsh:
                     continue
-                cond = "role == %d || role == %d" % (k, partner[k]) if k in partner else "role == %d" % k
-                fn = "arrow_local_m%d(role == %d ? 1 : 0, sJ, sL, sE, damping2, fac)" % (k, partner[k]) if k in partner else "arrow_local_w%d(sJ, sL, sE, damping2, fac)" % k
+                cond = "role == %d || role == %d" % (k - wsh, partner[k] - wsh) if k in partner else "role == %d" % (k - wsh)
+                fn = "arrow_local_m%d(role == %d ? 1 : 0, sJ, sL, sE, damping2, fac)" % (k, partner[k] - wsh) if k in partner else "arrow_local_w%d(sJ, sL, sE, damping2, fac)" % k
                 out.append("        if (%s) %s;" % (cond, fn))
             out.append("        sync();  // every role's contribution to the shared-column system is in the strip")
             out.append("        hook();")
             s_storer = None
             if self.spec.get("arrow_cap_solo"):
+                if folds:
+                    raise ValueError("fold_task: arrow_cap_solo is not supported")
                 # the small system on the solver role alone (the others wait at a second barrier instead of repeating it)
                 out.append("        if (role == %d) {" % solver)
                 out.extend(cap)
@@ -1815,23 +1943,23 @@ class Generator:
                 out.append("#pragma unroll")
                 out.append("            for (int i = 0; i < %d; ++i) s[i] = sL.get(%d + i);" % (A["ks"], A["soff"]))
                 out.append("        }")
-            elif not finishes[solver] and any(finishes[k] for k in range(len(groups)) if k != solver) and self.spec.get("arrow_solver_skips_cap", True):
+            elif not finishes[su] and any(finishes[k] for k in range(nu) if k != su) and self.spec.get("arrow_solver_skips_cap", True):
                 # The SOLVER role has no rows of its own to finish (no private columns): it needs s only for its step, which
                 # reads it from the strip behind the next barrier.  It skips the shared-column system, so its time between the
                 # two barriers belongs to the stop test, the ticket and the staged refill (dls_spec.cuh, kPrefetch) -- latency
                 # that used to sit in front of 400 instructions the other roles were running too.
-                s_storer = [k for k in range(len(groups)) if k != solver and finishes[k] and k not in A["mirror_of"]][0]
+                s_storer = [k for k in range(nu) if k != su and finishes[k] and k not in A["mirror_of"]][0] - wsh
                 out.append("        if (role != %d) {" % solver)
                 out.extend("    " + ln for ln in cap)
                 out.append("        }")
             else:
                 out.extend(cap)
             out.append("        IKB_PHASE_FENCE();")
-            for k in range(len(groups)):
+            for k in range(nu):
                 if k in A["mirror_of"] or not finishes[k]:
                     continue
-                cond = "role == %d || role == %d" % (k, partner[k]) if k in partner else "role == %d" % k
-                fn = "arrow_finish_m%d(role == %d ? 1 : 0, sJ, sL, sE, s, fac, y)" % (k, partner[k]) if k in partner else "arrow_finish_w%d(sJ, sL, sE, s, fac, y)" % k
+                cond = "role == %d || role == %d" % (k - wsh, partner[k] - wsh) if k in partner else "role == %d" % (k - wsh)
+                fn = "arrow_finish_m%d(role == %d ? 1 : 0, sJ, sL, sE, s, fac, y)" % (k, partner[k] - wsh) if k in partner else "arrow_finish_w%d(sJ, sL, sE, s, fac, y)" % k
                 out.append("        if (%s) %s;" % (cond, fn))
             if not self.spec.get("arrow_cap_solo"):
                 out.append("        if (role == %d) {" % (s_storer if s_storer is not None else solver))
@@ -1868,7 +1996,7 @@ class Generator:
         out.extend(integ)
         out.append("    }")
         if uniform or arrow:
-            C, roles, qsets = self.gen_step_roles_arrow(groups, solver) if arrow else self.gen_step_roles(groups, solver)
+            C, roles, qsets = self.gen_step_roles_arrow([g + folds for g in groups], solver) if arrow else self.gen_step_roles(groups, solver)
             out.append("    // Distributed step (see gen_step_roles): y from the strip; common joints by every role, the others by their role.")
             out.append("    template <typename T, typename S>")
             yreg = arrow and self.arrow["y_regs"]
