@@ -271,7 +271,8 @@ template <typename T> int launch_carry_tail(const ikb_problem *p, const CarrySta
 // Cassie-sized tree takes the smaller scratch of CoopClass<3> (dls_coop.cuh).  IKB_COOP_CLASS3=0 disables it (A/B runs).
 inline int coop_class(const ikb_problem *p) {
     const char *e = std::getenv("IKB_COOP_CLASS3");
-    if (p->size_class == 2 && p->hp.model.njoints() <= 20 && p->hp.model.nv <= 24 && !(e && e[0] == '0')) return 3;
+    const HostModel &m = p->hp.model;
+    if (p->size_class == 2 && m.njoints() <= 20 && m.nv <= 24 && m.nq <= 28 && !(e && e[0] == '0')) return 3;
     return p->size_class;
 }
 

@@ -9,7 +9,8 @@
 // compile-time alternative, through a double-buffered shared-memory column (SHFL = false; both measured, DESIGN.md).
 // Every phase of ik::dls (reference dls.cpp:14-74) is split by DATA over the lanes (SPMD, __syncwarp between phases):
 //
-//   phase 0  lane <-> joint: sin / cos of the revolute coordinates of the joints some task needs
+//   phase 0  lane <-> joint: sin / cos of the revolute coordinates of the joints some task needs (a continuous joint's
+//            q already holds them)
 //   phase 1  lane <-> (root-to-leaf path, row i): world placements by ROWS -- row i of R_world(j) and component i of
 //            p_world(j) depend only on row i of the parent's rotation, so a lane walks its path without communication,
 //            applying placement and joint motion on the fly                                     (data.cpp:28-29)
@@ -34,6 +35,7 @@
 #pragma once
 #include "../../include/ikb200.h"
 #include "dev_problem.hpp"
+#include "joint_types.hpp"
 #include "se3_math.cuh"
 
 namespace ikb {
@@ -63,7 +65,7 @@ template <> struct CoopClass<3> { using Cfg = CoopCfg<20, 24, 30, 32>; };
 // level costs residency, so a problem gets the smallest scratch that serves it.
 template <typename T, class Cfg, int EXTRA> struct alignas(16) CoopScratch {
     T Jt[Cfg::NV][Cfg::LD];   // weighted stacked task Jacobian, column-major; structural zeros are written once per kernel
-    T sc[Cfg::NJ][2];         // (sin, cos) of every needed revolute joint's coordinate
+    T sc[Cfg::NJ][2];         // (sin, cos) of every needed revolute or continuous joint's coordinate
     T oM[Cfg::NJ][12];        // oMi: R row-major (9) + p (3)
     T XY[Cfg::M][6];          // per task row: X (3), Y (3)
     T tpf[Cfg::M][3];         // per task: world origin of the task frame
@@ -78,7 +80,8 @@ template <typename T, class Cfg, int EXTRA> struct alignas(16) CoopScratch {
 };
 
 // World twist of velocity coordinate cc of joint j (data.cpp:30: oMi.act(S_i)) as (axis direction `ax`, origin `p`):
-// angular coordinates (revolute, free-flyer 3-5) give (v, w) = (p x ax, ax), linear ones (prismatic, free-flyer 0-2) (ax, 0).
+// angular coordinates (revolute, continuous, free-flyer 3-5) give (v, w) = (p x ax, ax), linear ones (prismatic, free-flyer
+// 0-2) (ax, 0).
 template <typename T> IKB_HD bool coop_world_axis(const DevProblem<T> &P, int j, int cc, const T *O, T *ax) {
     const int jt = P.jtype[j];
     if (jt == IKB_J_FREEFLYER) {
@@ -86,13 +89,13 @@ template <typename T> IKB_HD bool coop_world_axis(const DevProblem<T> &P, int j,
         ax[0] = O[k]; ax[1] = O[3 + k]; ax[2] = O[6 + k];
         return cc >= 3;
     }
-    const int k = (jt == IKB_J_RX || jt == IKB_J_PX) ? 0 : ((jt == IKB_J_RY || jt == IKB_J_PY) ? 1 : ((jt == IKB_J_RZ || jt == IKB_J_PZ) ? 2 : -1));
+    const int k = axis_index(jt);
     if (k >= 0) {
         ax[0] = O[k]; ax[1] = O[3 + k]; ax[2] = O[6 + k];
     } else {
         rot_vec(O, P.axis[j], ax);
     }
-    return jt <= IKB_J_REV_UNALIGNED;
+    return is_revolute_like(jt);
 }
 
 // World placement of used frame f (common.hpp:47-51: data.oMf[id]): oMi[parent] * placement, without the product when the
@@ -114,21 +117,24 @@ IKB_HD void coop_evaluate(const Ctx &cx, const DevProblem<T> &P, CoopScratch<T, 
     constexpr int TEAM = Cfg::TEAM;
     const CoopTables &C = P.coop;
     const int lane = cx.lane;
-    // phase 0: lane <-> joint, sin / cos of the revolute coordinates
+    // phase 0: lane <-> joint, sin / cos of the revolute coordinates; a continuous joint's q is (cos, sin) as given (Pinocchio's
+    // JointModelRevoluteUnbounded::calc neither evaluates nor renormalises it)
     for (int i = lane; i < C.n_fkj; i += TEAM) {
         const int j = C.fkj[i], t = P.jtype[j];
-        if (t >= IKB_J_RX && t <= IKB_J_REV_UNALIGNED) sincos_(S.q[P.idx_q[j]], &S.sc[j][0], &S.sc[j][1]);
+        if (is_revolute(t)) sincos_(S.q[P.idx_q[j]], &S.sc[j][0], &S.sc[j][1]);
+        else if (is_continuous(t)) { S.sc[j][0] = S.q[P.idx_q[j] + 1]; S.sc[j][1] = S.q[P.idx_q[j]]; }
     }
     cx.sync();
     // phase 1: lane <-> (path, row i).  oMi = oMi[parent] * placement * M_j(q) by rows: with r = row i of the parent's
     // rotation, a = r * placement.R is row i of (parent * placement) and the joint motion mixes two of its entries
-    // (aligned revolutes), multiplies it by the free-flyer's rotation, or leaves it alone (prismatic).
+    // (aligned revolutes), multiplies it by the free-flyer's rotation, or leaves it alone (prismatic).  A continuous joint
+    // moves as the revolute joint with its axis, from the (sin, cos) of phase 0.
     for (int w = lane; w < 3 * C.npaths; w += TEAM) {
         const int p = w / 3, i = w - 3 * p;
         T r0 = i == 0 ? T(1) : T(0), r1 = i == 1 ? T(1) : T(0), r2 = i == 2 ? T(1) : T(0), pp = T(0);
         const int len = C.path_len[p];
         for (int k = 0; k < len; ++k) {
-            const int j = C.path_joint[p][k], t = P.jtype[j];
+            const int j = C.path_joint[p][k], t = as_revolute(P.jtype[j]);
             const T *PR = P.placement[j];
             const T a0 = r0 * PR[0] + r1 * PR[3] + r2 * PR[6];
             const T a1 = r0 * PR[1] + r1 * PR[4] + r2 * PR[7];
@@ -734,6 +740,14 @@ IKB_HD T coop_iteration(const Ctx &cx, const DevProblem<T> &P, CoopScratch<T, Cf
                 quat_to_rot(S.q[iq + 3], S.q[iq + 4], S.q[iq + 5], S.q[iq + 6], R0);
                 integrate_freeflyer(R0, &S.q[iq], &S.q[iq + 3], v6);
                 for (int k = 0; k < 7; ++k) S.q[iq + k] = min_(P.upper[iq + k], max_(S.q[iq + k], P.lower[iq + k]));
+            } else if (is_continuous(jt)) {   // SpecialOrthogonalOperation<2>::integrate: rotate (c, s) by the step, first-order renormalisation
+                T sw, cw;
+                sincos_(step * S.dq[iv], &sw, &cw);
+                const T c0 = S.q[iq], s0 = S.q[iq + 1];
+                const T c1 = cw * c0 - sw * s0, s1 = sw * c0 + cw * s0;
+                const T a = (T(3) - (c1 * c1 + s1 * s1)) / T(2);
+                S.q[iq] = min_(P.upper[iq], max_(c1 * a, P.lower[iq]));
+                S.q[iq + 1] = min_(P.upper[iq + 1], max_(s1 * a, P.lower[iq + 1]));
             } else {
                 S.q[iq] = min_(P.upper[iq], max_(S.q[iq] + step * S.dq[iv], P.lower[iq]));
             }
@@ -756,6 +770,7 @@ template <typename T, class Cfg, int EXTRA, class Ctx> IKB_HD void coop_init_scr
         for (int i = 0; i < 12; ++i) S.oM[0][i] = (i % 4 == 0 && i < 9) ? T(1) : T(0);   // joint 0 = universe: identity, never recomputed
         for (int j = 1; j < P.njoints; ++j)
             if (P.jtype[j] == IKB_J_FREEFLYER) S.q[P.idx_q[j] + 6] = T(1);   // a team without a problem iterates on the neutral pose
+            else if (is_continuous(P.jtype[j])) S.q[P.idx_q[j]] = T(1);
         for (int t = 0; t < P.ntasks; ++t)
             if (P.t_kind[t] == IKB_TASK_POSTURE) {   // posture.hpp:60-66: J.rightCols(nj) = I (not masked), weighted (data.cpp:50)
                 const int nj = P.t_type[t], row = P.t_row[t];

@@ -17,6 +17,7 @@
 #include <cuda_runtime.h>
 
 #include "dev_problem.hpp"
+#include "joint_types.hpp"
 #include "se3_math.cuh"
 
 namespace ikb {
@@ -50,6 +51,17 @@ __device__ __forceinline__ void stage_blob_tma(void *smem_dst, const void *gmem_
     }
 }
 
+// unit axis of a revolute, continuous or prismatic joint in its own frame
+template <typename T>
+__device__ __forceinline__ void joint_axis_local(const DevProblem<T> &P, int j, T *a) {
+    const int t = as_revolute(P.jtype[j]);
+    a[0] = a[1] = a[2] = T(0);
+    if (t == IKB_J_RX || t == IKB_J_PX) a[0] = 1;
+    else if (t == IKB_J_RY || t == IKB_J_PY) a[1] = 1;
+    else if (t == IKB_J_RZ || t == IKB_J_PZ) a[2] = 1;
+    else { a[0] = P.axis[j][0]; a[1] = P.axis[j][1]; a[2] = P.axis[j][2]; }
+}
+
 // joint transform liMi = placement * M_j(q) for every joint type the flattener emits
 template <typename T>
 __device__ __forceinline__ void joint_local(const DevProblem<T> &P, int j, const T *q, T *Rl, T *pl) {
@@ -60,14 +72,16 @@ __device__ __forceinline__ void joint_local(const DevProblem<T> &P, int j, const
         T Rj[9];
         quat_to_rot(qj[3], qj[4], qj[5], qj[6], Rj);
         se3_mul(PR, Pp, Rj, qj, Rl, pl);
-    } else if (t >= IKB_J_RX && t <= IKB_J_REV_UNALIGNED) {
+    } else if (is_revolute_like(t)) {
         T s, c, Rj[9];
-        sincos_(qj[0], &s, &c);
-        if (t == IKB_J_RX) {
+        if (is_continuous(t)) { c = qj[0]; s = qj[1]; }   // (cos, sin) as given, not renormalised (RevoluteUnbounded::calc)
+        else sincos_(qj[0], &s, &c);
+        const int r = as_revolute(t);
+        if (r == IKB_J_RX) {
             Rj[0] = 1; Rj[1] = 0; Rj[2] = 0; Rj[3] = 0; Rj[4] = c; Rj[5] = -s; Rj[6] = 0; Rj[7] = s; Rj[8] = c;
-        } else if (t == IKB_J_RY) {
+        } else if (r == IKB_J_RY) {
             Rj[0] = c; Rj[1] = 0; Rj[2] = s; Rj[3] = 0; Rj[4] = 1; Rj[5] = 0; Rj[6] = -s; Rj[7] = 0; Rj[8] = c;
-        } else if (t == IKB_J_RZ) {
+        } else if (r == IKB_J_RZ) {
             Rj[0] = c; Rj[1] = -s; Rj[2] = 0; Rj[3] = s; Rj[4] = c; Rj[5] = 0; Rj[6] = 0; Rj[7] = 0; Rj[8] = 1;
         } else {
             const T *a = P.axis[j];
@@ -90,16 +104,6 @@ __device__ __forceinline__ void joint_local(const DevProblem<T> &P, int j, const
         for (int i = 0; i < 9; ++i) Rl[i] = PR[i];
         pl[0] = Pp[0] + o[0]; pl[1] = Pp[1] + o[1]; pl[2] = Pp[2] + o[2];
     }
-}
-
-template <typename T>
-__device__ __forceinline__ void joint_axis_local(const DevProblem<T> &P, int j, T *a) {
-    const int t = P.jtype[j];
-    a[0] = a[1] = a[2] = T(0);
-    if (t == IKB_J_RX || t == IKB_J_PX) a[0] = 1;
-    else if (t == IKB_J_RY || t == IKB_J_PY) a[1] = 1;
-    else if (t == IKB_J_RZ || t == IKB_J_PZ) a[2] = 1;
-    else { a[0] = P.axis[j][0]; a[1] = P.axis[j][1]; a[2] = P.axis[j][2]; }
 }
 
 // Forward kinematics of every joint (world placements), oR/op indexed by joint; joint 0 = universe = identity.
@@ -192,7 +196,7 @@ __device__ __forceinline__ void world_column(const DevProblem<T> &P, int j, int 
         T al[3], z[3];
         joint_axis_local(P, j, al);
         rot_vec(oR[j], al, z);
-        if (jt <= IKB_J_REV_UNALIGNED) { cross3(op[j], z, v); ww[0] = z[0]; ww[1] = z[1]; ww[2] = z[2]; }
+        if (is_revolute_like(jt)) { cross3(op[j], z, v); ww[0] = z[0]; ww[1] = z[1]; ww[2] = z[2]; }
         else { v[0] = z[0]; v[1] = z[1]; v[2] = z[2]; ww[0] = ww[1] = ww[2] = T(0); }
     }
 }
@@ -343,7 +347,7 @@ __global__ void __launch_bounds__(128) dls_generic_kernel(const DevProblem<T> *_
                                     T al[3], z[3];
                                     joint_axis_local(P, j, al);
                                     rot_vec(oR[j], al, z);
-                                    if (jt <= IKB_J_REV_UNALIGNED) { cross3(op[j], z, v); ww[0] = z[0]; ww[1] = z[1]; ww[2] = z[2]; }
+                                    if (is_revolute_like(jt)) { cross3(op[j], z, v); ww[0] = z[0]; ww[1] = z[1]; ww[2] = z[2]; }
                                     else { v[0] = z[0]; v[1] = z[1]; v[2] = z[2]; ww[0] = ww[1] = ww[2] = T(0); }
                                 }
                                 // oMf.actInv(column)
@@ -382,7 +386,7 @@ __global__ void __launch_bounds__(128) dls_generic_kernel(const DevProblem<T> *_
                         rotT_vec(Rm, rxt, r3);  // (r x t)^T R_rMf
                         for (int j = fj; j > 0; j = P.parent[j]) {
                             const int c0 = P.idx_v[j], jt = P.jtype[j];
-                            if (jt >= IKB_J_PX) continue;  // prismatic: no angular part
+                            if (is_prismatic(jt)) continue;  // no angular part
                             const int ncol = jt == IKB_J_FREEFLYER ? 6 : 1;
                             for (int cc = (jt == IKB_J_FREEFLYER ? 3 : 0); cc < ncol; ++cc) {
                                 T ww[3];
@@ -612,6 +616,13 @@ __global__ void __launch_bounds__(128) dls_generic_kernel(const DevProblem<T> *_
                         for (int i = 0; i < 6; ++i) v6[i] = a.step_length * dq[iv + i];
                         quat_to_rot(q[iq + 3], q[iq + 4], q[iq + 5], q[iq + 6], R0);
                         integrate_freeflyer(R0, &q[iq], &q[iq + 3], v6);
+                    } else if (is_continuous(P.jtype[j])) {   // SpecialOrthogonalOperation<2>::integrate
+                        T sw, cw;
+                        sincos_(a.step_length * dq[iv], &sw, &cw);
+                        const T c1 = cw * q[iq] - sw * q[iq + 1], s1 = sw * q[iq] + cw * q[iq + 1];
+                        const T al = (T(3) - (c1 * c1 + s1 * s1)) / T(2);
+                        q[iq] = c1 * al;
+                        q[iq + 1] = s1 * al;
                     } else {
                         q[iq] += a.step_length * dq[iv];
                     }

@@ -433,7 +433,7 @@ template <class Spec> bool spec_matches(const HostProblem &hp) {
     for (int j = 0; j < Spec::NJOINTS; ++j) {
         if (m.parent[j] != par[j] || m.jtype[j] != typ[j]) return false;
         if (!same_values(m.placement[j].data(), pl + 15 * j, 12)) return false;
-        if (typ[j] == IKB_J_REV_UNALIGNED || typ[j] == IKB_J_PRIS_UNALIGNED)
+        if (typ[j] > IKB_J_FREEFLYER && axis_index(typ[j]) < 0)   // unaligned: the axis is part of the model
             if (!same_values(m.axis[j].data(), pl + 15 * j + 12, 3)) return false;
     }
     // tasks must already be in stacked order (the generated code has no notion of insertion order)
@@ -486,7 +486,7 @@ template <class Spec> bool spec_near_miss(const HostProblem &hp, std::string *wh
     const double *pl = Spec::sig_placement();
     for (int j = 0; j < Spec::NJOINTS; ++j) {
         scan(m.placement[j].data(), pl + 15 * j, 12, "placement of joint", j, m.joint_names[j].c_str());
-        if (typ[j] == IKB_J_REV_UNALIGNED || typ[j] == IKB_J_PRIS_UNALIGNED) scan(m.axis[j].data(), pl + 15 * j + 12, 3, "axis of joint", j, m.joint_names[j].c_str());
+        if (typ[j] > IKB_J_FREEFLYER && axis_index(typ[j]) < 0) scan(m.axis[j].data(), pl + 15 * j + 12, 3, "axis of joint", j, m.joint_names[j].c_str());
     }
     for (int t = 0; t < Spec::NTASKS; ++t) {
         const HostTask &ht = hp.tasks[t];

@@ -203,7 +203,7 @@ int ikb_model_from_desc(const ikb_model_desc *d, ikb_model **out) {
     int iq = 0;
     for (int j = 0; j < d->njoints; ++j) {
         const int t = d->jtype[j];
-        if (t < IKB_J_UNIVERSE || t > IKB_J_PRIS_UNALIGNED || (j > 0 && (d->parent[j] < 0 || d->parent[j] >= j))) {
+        if (t < IKB_J_UNIVERSE || t > IKB_J_RUB_UNALIGNED || (j > 0 && (d->parent[j] < 0 || d->parent[j] >= j))) {
             delete h;
             return fail(IKB_ERR_INVALID_ARG, "ikb_model_from_desc: bad joint type or parent index (parents must precede children)");
         }
@@ -211,7 +211,7 @@ int ikb_model_from_desc(const ikb_model_desc *d, ikb_model **out) {
         std::copy(d->placement + 12 * j, d->placement + 12 * j + 12, pl.begin());
         std::array<double, 3> ax{0, 0, 0};
         if (d->axis) ax = {d->axis[3 * j], d->axis[3 * j + 1], d->axis[3 * j + 2]};
-        const int n = HostModel::joint_nq(t);
+        const int n = joint_nq(t);
         std::vector<double> lo(n), hi(n);
         for (int k = 0; k < n; ++k) {
             lo[k] = d->lower ? d->lower[iq + k] : -1e300;
@@ -295,6 +295,7 @@ int ikb_model_neutral(const ikb_model *m, double *q) {
     std::fill(q, q + m->m.nq, 0.0);
     for (int j = 0; j < m->m.njoints(); ++j)
         if (m->m.jtype[j] == IKB_J_FREEFLYER) q[m->m.idx_q[j] + 6] = 1.0;
+        else if (is_continuous(m->m.jtype[j])) q[m->m.idx_q[j]] = 1.0;   // (cos, sin) = (1, 0)
     return IKB_OK;
 }
 
@@ -374,7 +375,15 @@ int ikb_problem_add_align_axis_task(ikb_problem *p, int frame, int axis, int ref
 
 int ikb_problem_add_posture_task(ikb_problem *p, int nj, int priority, const double *weights, const double *mask) {
     if (!p) return -fail(IKB_ERR_INVALID_ARG, "null problem");
-    if (nj < 1 || nj > p->hp.model.nv || nj > p->hp.model.nq) return -fail(IKB_ERR_INVALID_ARG, "posture size out of range");
+    const HostModel &m = p->hp.model;
+    if (nj < 1 || nj > m.nv || nj > m.nq) return -fail(IKB_ERR_INVALID_ARG, "posture size out of range");
+    // posture.hpp:50-67 pairs q.tail(nj) with the last nj velocity coordinates: with a continuous joint (two entries of q,
+    // one of v) among those, they no longer name the same joints
+    for (int j = 1; j < m.njoints(); ++j)
+        if (is_continuous(m.jtype[j]) && m.idx_v[j] >= m.nv - nj)
+            return -fail(IKB_ERR_UNSUPPORTED, "posture task over the last " + std::to_string(nj) + " coordinates: joint " +
+                                                  m.joint_names[j] + " among them is continuous, so q.tail(nj) and the last nj "
+                                                  "velocity coordinates would not name the same joints");
     HostTask t;
     t.kind = IKB_TASK_POSTURE;
     t.type = nj;
@@ -462,13 +471,13 @@ int ikb_problem_finalize(ikb_problem *p, int device) {
         hp.rows() > kMaxRows)
         return fail(IKB_ERR_UNSUPPORTED, "problem exceeds the compiled capacities of the constant blob");
     int cls = -1;
-    for (int c = 0; c < 3; ++c)
-        if (m.njoints() <= kClasses[c].nj && m.nv <= kClasses[c].nv && hp.rows() <= kClasses[c].m) {
+    for (int c = 0; c < 3; ++c)   // the kernels size q as nv + 4 scalars (continuous joints make nq exceed nv)
+        if (m.njoints() <= kClasses[c].nj && m.nv <= kClasses[c].nv && m.nq <= kClasses[c].nv + 4 && hp.rows() <= kClasses[c].m) {
             cls = c;
             break;
         }
     if (cls < 0)
-        return fail(IKB_ERR_UNSUPPORTED, "problem larger than the generic kernel's largest size class (32 joints, nv 36, 30 rows)");
+        return fail(IKB_ERR_UNSUPPORTED, "problem larger than the generic kernel's largest size class (32 joints, nv 36, nq 40, 30 rows)");
 
     int ndev = 0;
     cudaError_t e = cudaGetDeviceCount(&ndev);

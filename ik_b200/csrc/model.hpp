@@ -11,6 +11,7 @@
 #include <vector>
 
 #include "../../include/ikb200.h"
+#include "joint_types.hpp"
 
 namespace ikb {
 
@@ -42,8 +43,6 @@ struct HostModel {
     int add_joint(const std::string &name, int type, int parent_joint, const SE3d &pl, const std::array<double, 3> &ax,
                   const std::vector<double> &lo, const std::vector<double> &hi);
     int add_frame(const std::string &name, int parent_joint, const SE3d &pl, int type);
-    static int joint_nq(int type) { return type == IKB_J_UNIVERSE ? 0 : (type == IKB_J_FREEFLYER ? 7 : 1); }
-    static int joint_nv(int type) { return type == IKB_J_UNIVERSE ? 0 : (type == IKB_J_FREEFLYER ? 6 : 1); }
 };
 
 // URDF text -> HostModel following urdfdom + Pinocchio's traversal (SURVEY.md 8c.1).  Throws

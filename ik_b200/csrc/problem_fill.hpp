@@ -93,7 +93,7 @@ inline bool build_coop_tables(const HostProblem &hp, const std::vector<int> &ord
         else
             for (int j = m.frame_parent[t.frame]; j > 0; j = m.parent[j]) joints.push_back(j);
         for (int j : joints)
-            for (int cc = 0; cc < HostModel::joint_nv(m.jtype[j]); ++cc) {
+            for (int cc = 0; cc < joint_nv(m.jtype[j]); ++cc) {
                 if (C.npairs >= kCoopMaxPairs) return false;
                 C.pair_task[C.npairs] = (uint8_t)s;
                 C.pair_joint[C.npairs] = (uint8_t)j;
@@ -167,7 +167,7 @@ inline void fill_dev_problem(const HostProblem &hp, const std::vector<int> &orde
             cols = m.nv >= 64 ? ~0ULL : ((1ULL << m.nv) - 1);
         } else {
             for (int j = m.frame_parent[t.frame]; j > 0; j = m.parent[j])
-                for (int k = 0; k < HostModel::joint_nv(m.jtype[j]); ++k) cols |= 1ULL << (m.idx_v[j] + k);
+                for (int k = 0; k < joint_nv(m.jtype[j]); ++k) cols |= 1ULL << (m.idx_v[j] + k);
         }
         for (int i = 0; i < t.dim; ++i) {
             P.row_cols[row + i] = cols;

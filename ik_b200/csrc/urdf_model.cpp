@@ -5,7 +5,8 @@
 //     std::map<std::string, ...>), the tree is walked depth-first, movable joints are numbered in visit
 //     order, fixed joints collapse into frames on the supporting joint;
 //   * rpy -> quaternion (urdfdom Rotation::setFromRPY, normalised) -> matrix (Eigen), literals verbatim;
-//   * a unit axis selects RX/RY/RZ (PX/PY/PZ), anything else is an unaligned joint with a normalised axis;
+//   * a unit axis selects RX/RY/RZ (PX/PY/PZ, RUBX/RUBY/RUBZ), anything else is an unaligned joint with a normalised axis;
+//   * a continuous joint is Pinocchio's unbounded revolute: q = (cos, sin), both entries bounded by +-1.01;
 //   * the optional free-flyer root joint is "root_joint" with limits +-DBL_MAX.
 // The XML reader below is a minimal non-validating parser (elements, attributes, comments, PIs, CDATA).
 #include <cfloat>
@@ -284,14 +285,15 @@ struct Builder {
         if (j.type == "fixed") {
             m.add_frame(j.name, support, placement, FRAME_FIXED_JOINT);
             body_frame[j.child] = m.add_frame(j.child, support, placement, FRAME_BODY);
-        } else if (j.type == "revolute" || j.type == "prismatic") {
-            const bool rev = j.type == "revolute";
-            int type = rev ? IKB_J_REV_UNALIGNED : IKB_J_PRIS_UNALIGNED;
+        } else if (j.type == "revolute" || j.type == "prismatic" || j.type == "continuous") {
+            const bool rev = j.type == "revolute", cont = j.type == "continuous";
+            const int first = rev ? IKB_J_RX : (cont ? IKB_J_RUBX : IKB_J_PX);   // X, Y, Z, unaligned follow in that order
+            int type = first + 3;
             std::array<double, 3> ax = j.axis;
             bool aligned = false;
             for (int k = 0; k < 3 && !aligned; ++k)
                 if (approx_unit(j.axis, k)) {
-                    type = (rev ? IKB_J_RX : IKB_J_PX) + k;
+                    type = first + k;
                     ax = {0, 0, 0};
                     ax[k] = 1.0;
                     aligned = true;
@@ -301,7 +303,9 @@ struct Builder {
                 if (!(n > 0)) throw std::runtime_error("URDF: joint " + j.name + " has a zero axis");
                 for (auto &v : ax) v /= n;
             }
-            const int jid = m.add_joint(j.name, type, support, placement, ax, {j.lower}, {j.upper});
+            // continuous: Pinocchio's URDF parser bounds both entries of (cos, sin) by -1.01 / +1.01 and ignores <limit>
+            const int jid = cont ? m.add_joint(j.name, type, support, placement, ax, {-1.01, -1.01}, {1.01, 1.01})
+                                 : m.add_joint(j.name, type, support, placement, ax, {j.lower}, {j.upper});
             m.add_frame(j.name, jid, se3_identity(), FRAME_JOINT);
             body_frame[j.child] = m.add_frame(j.child, jid, se3_identity(), FRAME_BODY);
         } else {

@@ -1,8 +1,9 @@
 """Synthetic IK workloads of BASELINE.json (SURVEY.md 8d), generated identically for the CPU oracle and the GPU.
 
 Per problem b (counter-based SplitMix64 keyed by (seed, b, k), so any shard of a batch can be generated
-independently): a reachable configuration q* with revolute joints uniform inside the URDF limits, base
-position uniform in [-0.2, 0.2]^3 m and base orientation exp3(u), u uniform in [-0.3, 0.3]^3 rad; the task
+independently): a reachable configuration q* with revolute joints uniform inside the URDF limits, continuous
+joints at an angle uniform in [-pi, pi) (q = (cos, sin)), base position uniform in [-0.2, 0.2]^3 m and base
+orientation exp3(u), u uniform in [-0.3, 0.3]^3 rad; the task
 targets are the task frames' placements at q* expressed in ``universe``.  Position tasks get the target
 (Identity, p) -- the reference's FrameTask keeps ``target`` at se3_t::Identity() and callers only set the
 translation (ik_ros/src/cassie.cpp:95-96).  The initial guess is the SRDF standing pose with an identity base.
@@ -17,6 +18,7 @@ CASSIE_STANDING = [0.0045, 0.0, 0.4973, -1.1997, 0.0, 1.4267, 0.0, -1.5968,
                    -0.0045, 0.0, 0.4973, -1.1997, 0.0, 1.4267, 0.0, -1.5968]
 
 J_FREEFLYER = 1
+J_CONTINUOUS = (10, 11, 12, 13)   # IKB_J_RUBX .. IKB_J_RUB_UNALIGNED: q = (cos theta, sin theta)
 
 _M64 = np.uint64(0xFFFFFFFFFFFFFFFF)
 
@@ -56,6 +58,10 @@ def sample_configurations(model, B, seed=12345, b0=0, margin=0.0):
             s = np.where(th > 1e-12, np.sin(th / 2) / np.maximum(th, 1e-300), 0.5)
             q[:, iq + 3:iq + 6] = u * s[:, None]
             q[:, iq + 6] = np.cos(th / 2)
+        elif model.jtypes[j] in J_CONTINUOUS:   # theta ~ U[-pi, pi): a continuous joint has no limits to sample inside
+            th = -np.pi + 2 * np.pi * uniform01(seed, b, k)
+            k += 1
+            q[:, iq], q[:, iq + 1] = np.cos(th), np.sin(th)
         else:
             w = hi[iq] - lo[iq]
             q[:, iq] = lo[iq] + margin * w + (1 - 2 * margin) * w * uniform01(seed, b, k)
@@ -72,8 +78,8 @@ def standing_configuration(model, standing=None):
 
 def near_start(model, qstar, seed=12345, b0=0, radius=0.3):
     """Warm-start initial guesses (the reference's only caller warm-starts every solve, ik_ros/src/cassie.cpp:112):
-    revolute joints = q* + U[-radius, radius] clipped to the limits, floating base at the identity.  Used for the
-    robots that have no SRDF standing pose; starting the serial arm at its singular zero configuration with full
+    revolute joints = q* + U[-radius, radius] clipped to the limits, continuous joints at the angle of q* plus
+    U[-radius, radius], floating base at the identity.  Used for the robots that have no SRDF standing pose; starting the serial arm at its singular zero configuration with full
     undamped-ish steps gives chaotic trajectories on which no two floating-point implementations agree."""
     B = qstar.shape[0]
     b = np.arange(b0, b0 + B, dtype=np.uint64)
@@ -86,7 +92,11 @@ def near_start(model, qstar, seed=12345, b0=0, radius=0.3):
             continue
         d = -radius + 2 * radius * uniform01(seed, b, k)
         k += 1
-        q0[:, iq] = np.minimum(hi[iq], np.maximum(lo[iq], qstar[:, iq] + d))
+        if model.jtypes[j] in J_CONTINUOUS:   # perturb the angle of (cos, sin); the pair stays a unit vector, nothing to clip
+            th = np.arctan2(qstar[:, iq + 1], qstar[:, iq]) + d
+            q0[:, iq], q0[:, iq + 1] = np.cos(th), np.sin(th)
+        else:
+            q0[:, iq] = np.minimum(hi[iq], np.maximum(lo[iq], qstar[:, iq] + d))
     return q0
 
 

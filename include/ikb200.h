@@ -41,10 +41,13 @@ typedef enum {
     IKB_ERR_NOT_FINALIZED = 7
 } ikb_status;
 
-/* joint types of the flattened tree (Pinocchio JointModel* equivalents) */
+/* joint types of the flattened tree (Pinocchio JointModel* equivalents).  RUB* are URDF `continuous` joints
+ * (JointModelRevoluteUnbounded{X,Y,Z} / ...Unaligned): two configuration entries (cos theta, sin theta) and one velocity
+ * coordinate; every other movable joint has one of each except the free-flyer (7 / 6). */
 typedef enum {
     IKB_J_UNIVERSE = 0, IKB_J_FREEFLYER = 1, IKB_J_RX = 2, IKB_J_RY = 3, IKB_J_RZ = 4, IKB_J_REV_UNALIGNED = 5,
-    IKB_J_PX = 6, IKB_J_PY = 7, IKB_J_PZ = 8, IKB_J_PRIS_UNALIGNED = 9
+    IKB_J_PX = 6, IKB_J_PY = 7, IKB_J_PZ = 8, IKB_J_PRIS_UNALIGNED = 9,
+    IKB_J_RUBX = 10, IKB_J_RUBY = 11, IKB_J_RUBZ = 12, IKB_J_RUB_UNALIGNED = 13
 } ikb_joint_type;
 
 /* ik::KinematicType, reference ik/ik/frame.hpp:20 */
@@ -106,7 +109,7 @@ int ikb_model_get_placements(const ikb_model *m, double *placement /*[njoints][1
 int ikb_model_get_limits(const ikb_model *m, double *lower, double *upper);
 int ikb_model_set_limits(ikb_model *m, const double *lower, const double *upper);
 int ikb_model_get_frames(const ikb_model *m, int32_t *parent_joint, int32_t *type, double *placement /*[nframes][12]*/);
-int ikb_model_neutral(const ikb_model *m, double *q); /* pinocchio::neutral: zeros, unit quaternion */
+int ikb_model_neutral(const ikb_model *m, double *q); /* pinocchio::neutral: zeros, unit quaternion, (1, 0) for continuous joints */
 
 /* ---- problem (host only until finalize) --------------------------------------------------------- */
 /* InverseKinematicsProblem(model, max_priority_level), reference problem.hpp:17-22 (copies the model) */
@@ -120,7 +123,9 @@ int ikb_problem_add_frame_task(ikb_problem *p, int frame, int kinematic_type, in
 /* AlignAxisTask + add_align_axis_task: frame.hpp:210-319, problem.hpp:94-105 */
 int ikb_problem_add_align_axis_task(ikb_problem *p, int frame, int axis, int reference_frame, int priority,
                                     const double *weights);
-/* PostureTask(model, nj) + add_posture_task: posture.hpp:17-86, problem.hpp:134-145.  mask: nj entries or NULL */
+/* PostureTask(model, nj) + add_posture_task: posture.hpp:17-86, problem.hpp:134-145.  mask: nj entries or NULL.
+ * IKB_ERR_UNSUPPORTED when a continuous joint has one of the last nj velocity coordinates (q.tail(nj) and the last nj
+ * columns would not name the same joints). */
 int ikb_problem_add_posture_task(ikb_problem *p, int nj, int priority, const double *weights, const double *mask);
 /* CentreOfMassTask (reference centre_of_mass.hpp:14-52, problem.hpp add_centre_of_mass_task, data.cpp:31-34):
  * e = oMr^-1 com(q) - target, J = R_r^T Jcom; 3 rows, target = 3 scalars.  Needs link masses: models from URDF read

@@ -31,7 +31,9 @@ import json
 import re
 import sys
 
-J_UNIVERSE, J_FF, J_RX, J_RY, J_RZ, J_RU, J_PX, J_PY, J_PZ, J_PU = range(10)
+J_UNIVERSE, J_FF, J_RX, J_RY, J_RZ, J_RU, J_PX, J_PY, J_PZ, J_PU, J_CX, J_CY, J_CZ, J_CU = range(14)
+J_CONT = (J_CX, J_CY, J_CZ, J_CU)   # continuous (RevoluteUnbounded): q = (cos, sin), the revolute's motion about the same axis
+J_REV = (J_RX, J_RY, J_RZ, J_RU) + J_CONT
 POSITION, ORIENTATION, FULL = 0, 1, 2
 
 
@@ -157,6 +159,12 @@ class Generator:
         self.joints = model["joints"]
         self.frames = {f["name"]: f for f in model["frames"]}
         self.nq, self.nv = model["nq"], model["nv"]
+        if any(j["type"] in J_CONT for j in self.joints):
+            # these options address the configuration as one scalar per joint (mirror's side-dependent qm registers) or
+            # were built for Cassie's free-flyer and revolute legs only
+            for opt in ("mirror", "fold_task", "tmem_j"):
+                if spec.get(opt) or (opt == "fold_task" and spec.get(opt) is not None):   # (fold_task is a task index)
+                    raise ValueError("spec option %r does not support continuous joints" % opt)
         self.tasks = []
         row = 0
         toff = 0
@@ -250,9 +258,13 @@ class Generator:
             R = matmul(E, A, Rq, "R%d" % j)
             p = matvec(E, A, ["q[%d]" % self.ql(iq + k) for k in range(3)], "p%d" % j, add=p)
             w = dict(R=R, p=p, z=None, type=t)
-        elif t in (J_RX, J_RY, J_RZ, J_RU):
-            E.raw("T s%d, c%d;" % (j, j))
-            E.raw("sincos_(%s, &s%d, &c%d);" % (self.qref(j, iq), j, j))
+        elif t in J_REV:
+            if t in J_CONT:   # (cos, sin) as given: no sin / cos evaluated, no renormalisation (RevoluteUnbounded::calc)
+                E.raw("const T c%d = q[%d], s%d = q[%d];" % (j, self.ql(iq), j, self.ql(iq + 1)))
+                t = J_RX + J_CONT.index(t)
+            else:
+                E.raw("T s%d, c%d;" % (j, j))
+                E.raw("sincos_(%s, &s%d, &c%d);" % (self.qref(j, iq), j, j))
             s, c = "s%d" % j, "c%d" % j
             if t == J_RU:
                 a = jt["axis"]
@@ -522,7 +534,7 @@ class Generator:
                         if bot:
                             for i in range(3):
                                 store(brow + i, iv + 3 + k, neg(E, m1r[i]))
-                elif jt["type"] in (J_RX, J_RY, J_RZ, J_RU):
+                elif jt["type"] in J_REV:
                     z = w["z"]
                     m1z = matvec(E, M1, z, "m1z")
                     if top:
@@ -587,7 +599,7 @@ class Generator:
                     rk = [w["R"][k], w["R"][3 + k], w["R"][6 + k]]
                     d = sop(E, [(u[i], rk[i]) for i in range(3)], "al")
                     E.raw("sJ.set(%d, c.weight[%d] * -(%s));  // J[%d][%d]" % (self.slot(row, iv + 3 + k), row, lit(d), row, iv + 3 + k))
-            elif jt["type"] in (J_RX, J_RY, J_RZ, J_RU):
+            elif jt["type"] in J_REV:
                 d = sop(E, [(u[i], w["z"][i]) for i in range(3)], "al")
                 E.raw("sJ.set(%d, c.weight[%d] * -(%s));  // J[%d][%d]" % (self.slot(row, iv), row, lit(d), row, iv))
             # prismatic joints have no angular part
@@ -1573,7 +1585,7 @@ class Generator:
         cols, qs = [], []
         for j in joints:
             jt = self.joints[j]
-            nvj, nqj = (6, 7) if jt["type"] == J_FF else (1, 1)
+            nvj, nqj = (6, 7) if jt["type"] == J_FF else ((1, 2) if jt["type"] in J_CONT else (1, 1))
             cols.extend(range(jt["idx_v"], jt["idx_v"] + nvj))
             qs.extend(range(jt["idx_q"], jt["idx_q"] + nqj))
         return cols, qs
@@ -1613,6 +1625,16 @@ class Generator:
                 if [self.ql(iq + k) for k in range(7)] != list(range(self.ql(iq), self.ql(iq) + 7)):
                     raise ValueError("free-flyer coordinates must be contiguous in the local registers")
                 L.append(ind + "    integrate_freeflyer(R0, &q[%d], &q[%d], v6);" % (self.ql(iq), self.ql(iq + 3)))
+                L.append(ind + "}")
+            elif jt["type"] in J_CONT:   # SpecialOrthogonalOperation<2>::integrate: rotate (c, s), first-order renormalisation
+                c0, s0 = self.ql(iq), self.ql(iq + 1)
+                L.append(ind + "{")
+                L.append(ind + "    T sw, cw;")
+                L.append(ind + "    sincos_(step * dq[%d], &sw, &cw);" % iv)
+                L.append(ind + "    const T c1 = cw * q[%d] - sw * q[%d], s1 = sw * q[%d] + cw * q[%d];" % (c0, s0, c0, s0))
+                L.append(ind + "    const T al = (T(3) - (c1 * c1 + s1 * s1)) / T(2);")
+                L.append(ind + "    q[%d] = c1 * al;" % c0)
+                L.append(ind + "    q[%d] = s1 * al;" % s0)
                 L.append(ind + "}")
             else:
                 L.append(ind + "q[%d] += step * dq[%d];" % (self.ql(iq), iv))
