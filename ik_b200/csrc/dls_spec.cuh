@@ -88,6 +88,7 @@ template <class Spec, typename T> constexpr int spec_tmem_cols(int nwarps) {
     return m <= 32 ? 32 : m <= 64 ? 64 : m <= 128 ? 128 : m <= 256 ? 256 : 512;
 }
 
+// (ik_b200/specialise.py spec_launch restates this to refuse, in words, a plugin spec that does not fit)
 template <class Spec, typename T> struct SpecLaunch {
     static constexpr int NW = Spec::NWARPS;
     static constexpr bool kTmemJ = spec_tmem_j<Spec, T>();
@@ -423,6 +424,14 @@ inline bool same_values(const double *a, const double *b, int n) {  // value equ
     return true;
 }
 
+// Specs with a centre-of-mass task fold every joint's mass and centre of mass into their code and carry them as
+// Spec::sig_inertia() (mass, com x, y, z per joint); the other generated headers have no such member.
+template <class Spec, class = void> struct spec_has_inertia : std::false_type {};
+template <class Spec> struct spec_has_inertia<Spec, std::void_t<decltype(Spec::sig_inertia())>> : std::true_type {};
+
+// generator task kind code (sig_task_kind) -> HostTask::kind
+constexpr int kSpecTaskKinds[4] = {IKB_TASK_FRAME, IKB_TASK_ALIGN_AXIS, IKB_TASK_POSTURE, IKB_TASK_COM};
+
 // Does the finalized problem equal the (tree, task list) this specialisation was generated for?
 template <class Spec> bool spec_matches(const HostProblem &hp) {
     const HostModel &m = hp.model;
@@ -436,15 +445,23 @@ template <class Spec> bool spec_matches(const HostProblem &hp) {
         if (typ[j] > IKB_J_FREEFLYER && axis_index(typ[j]) < 0)   // unaligned: the axis is part of the model
             if (!same_values(m.axis[j].data(), pl + 15 * j + 12, 3)) return false;
     }
+    // the inertias the com task's code was generated with (ikb_model_set_inertias).  Every joint is compared, the massless
+    // `universe` (joint 0) too, although no centre of mass reads its entry: tools/com_plugin_bench.py tells two plugins of
+    // one task list apart by it.
+    if constexpr (spec_has_inertia<Spec>::value) {
+        const double *in = Spec::sig_inertia();
+        for (int j = 0; j < Spec::NJOINTS; ++j)
+            if (!(m.mass[j] == in[4 * j]) || !same_values(m.com[j].data(), in + 4 * j + 1, 3)) return false;
+    }
     // tasks must already be in stacked order (the generated code has no notion of insertion order)
     for (int t = 0; t < Spec::NTASKS; ++t) {
         const HostTask &ht = hp.tasks[t];
-        const int kinds[3] = {IKB_TASK_FRAME, IKB_TASK_ALIGN_AXIS, IKB_TASK_POSTURE};
-        if (ht.kind != kinds[Spec::sig_task_kind()[t]]) return false;
+        if (ht.kind != kSpecTaskKinds[Spec::sig_task_kind()[t]]) return false;
         if (ht.type != Spec::sig_task_type()[t] || ht.priority != Spec::sig_task_priority()[t]) return false;  // type / axis / nj
         if (t > 0 && ht.priority < hp.tasks[t - 1].priority) return false;
         if (ht.kind == IKB_TASK_POSTURE) continue;  // no frames
         // the reference frame (`universe` or a moving frame) and the task frame must sit where the generator saw them
+        // (a centre-of-mass task has no frame of its own: HostTask::frame is its reference frame)
         if (m.frame_parent[ht.ref] != Spec::sig_task_ref_joint()[t]) return false;
         if (!same_values(m.frame_placement[ht.ref].data(), Spec::sig_task_ref_placement() + 12 * t, 12)) return false;
         if (m.frame_parent[ht.frame] != Spec::sig_task_joint()[t]) return false;
@@ -464,10 +481,9 @@ template <class Spec> bool spec_near_miss(const HostProblem &hp, std::string *wh
     const int *par = Spec::sig_parent(), *typ = Spec::sig_type();
     for (int j = 0; j < Spec::NJOINTS; ++j)
         if (m.parent[j] != par[j] || m.jtype[j] != typ[j]) return false;
-    const int kinds[3] = {IKB_TASK_FRAME, IKB_TASK_ALIGN_AXIS, IKB_TASK_POSTURE};
     for (int t = 0; t < Spec::NTASKS; ++t) {
         const HostTask &ht = hp.tasks[t];
-        if (ht.kind != kinds[Spec::sig_task_kind()[t]] || ht.type != Spec::sig_task_type()[t] || ht.priority != Spec::sig_task_priority()[t]) return false;
+        if (ht.kind != kSpecTaskKinds[Spec::sig_task_kind()[t]] || ht.type != Spec::sig_task_type()[t] || ht.priority != Spec::sig_task_priority()[t]) return false;
         if (ht.kind == IKB_TASK_POSTURE) continue;
         if (m.frame_parent[ht.ref] != Spec::sig_task_ref_joint()[t] || m.frame_parent[ht.frame] != Spec::sig_task_joint()[t]) return false;
     }

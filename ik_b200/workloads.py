@@ -10,8 +10,8 @@ translation (ik_ros/src/cassie.cpp:95-96).  The initial guess is the SRDF standi
 """
 import numpy as np
 
-from .api import (AlignAxisTask, AlignAxisType, FrameTask, InverseKinematicsProblem, KinematicType, Model,
-                  PostureTask)
+from .api import (AlignAxisTask, AlignAxisType, CentreOfMassTask, FrameTask, InverseKinematicsProblem, KinematicType,
+                  Model, PostureTask)
 
 # cassie-description/srdf/cassie.srdf:22-39 (group_state "default"), in model joint order
 CASSIE_STANDING = [0.0045, 0.0, 0.4973, -1.1997, 0.0, 1.4267, 0.0, -1.5968,
@@ -156,6 +156,35 @@ def cassie_demo_posture_problem(model=None):
     return pb
 
 
+def cassie_com_problem(model=None, reference="universe"):
+    """Cassie balancing: LeftFootFront Position, the centre of mass (CentreOfMassTask in `reference`), RightFootFront Position
+    and the pelvis Orientation, all on level 0 -- 12 task rows.  Set the centre-of-mass target with com_targets()."""
+    model = model or cassie_model()
+    pb = InverseKinematicsProblem(model, 0)
+    pb.add_frame_task("fl", FrameTask(model, "LeftFootFront", KinematicType.Position))
+    pb.add_centre_of_mass_task(CentreOfMassTask(model, reference))
+    pb.add_frame_task("fr", FrameTask(model, "RightFootFront", KinematicType.Position))
+    pb.add_frame_task("pelvis", FrameTask(model, "pelvis", KinematicType.Orientation))
+    return pb
+
+
+def com_targets(problem, targets, coms, poses=None):
+    """Set the target of the problem's CentreOfMassTask in `targets` [B, tsz] (in place; returned): coms [B, 3] are the world
+    centres of mass at the configurations q* the other targets come from (the oracle's center_of_mass, say), expressed here
+    in the task's reference frame, whose world placement poses[frame] [B, 12] supplies (task_frames lists it), so that q*
+    reaches every target."""
+    task = problem.get_centre_of_mass_task()
+    if task is None:
+        return targets
+    c = np.asarray(coms, dtype=np.float64)
+    if task.reference_frame != "universe":
+        Mr = poses[task.reference_frame]
+        c = np.einsum("bji,bj->bi", Mr[:, :9].reshape(-1, 3, 3), c - Mr[:, 9:12])
+    off = problem.target_offset(task)
+    targets[:, off:off + 3] = c
+    return targets
+
+
 def frame_task_list(problem):
     return [(t, problem.target_offset(t)) for _, t, _ in problem._tasks if isinstance(t, FrameTask)]
 
@@ -195,11 +224,11 @@ def targets_from_frame_poses(problem, poses, qstar=None):
 
 
 def task_frames(problem):
-    """Frames whose placements targets_from_frame_poses needs."""
+    """Frames whose placements targets_from_frame_poses and com_targets need."""
     names = []
     for _, t, _ in problem._tasks:
-        if isinstance(t, (FrameTask, AlignAxisTask)):
-            for n in (t.frame, t.reference_frame):
+        if isinstance(t, (FrameTask, AlignAxisTask, CentreOfMassTask)):
+            for n in (t.reference_frame,) if isinstance(t, CentreOfMassTask) else (t.frame, t.reference_frame):
                 if n != "universe" and n not in names:
                     names.append(n)
     return names

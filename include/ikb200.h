@@ -130,7 +130,9 @@ int ikb_problem_add_posture_task(ikb_problem *p, int nj, int priority, const dou
 /* CentreOfMassTask (reference centre_of_mass.hpp:14-52, problem.hpp add_centre_of_mass_task, data.cpp:31-34):
  * e = oMr^-1 com(q) - target, J = R_r^T Jcom; 3 rows, target = 3 scalars.  Needs link masses: models from URDF read
  * <inertial><mass>/<origin xyz>; ikb_model_set_inertias supplies them for models built from flat arrays.  Runs on
- * the table-driven kernel.  Returns the task index (insertion order) or minus an ikb_status. */
+ * the table-driven kernel unless a loaded plugin matches (ikb_load_specialisation; a plugin folds the model's masses and
+ * centres of mass into its code, so it matches only problems whose model still carries those inertias).  Returns the
+ * task index (insertion order) or minus an ikb_status. */
 int ikb_problem_add_com_task(ikb_problem *p, int ref, int priority, const double *weights /* 3 or NULL */);
 /* per joint: mass of the bodies it supports and their centre of mass in the joint frame (Pinocchio inertias[j]) */
 int ikb_model_get_inertias(const ikb_model *m, double *mass /* [njoints] */, double *com /* [njoints][3] */);

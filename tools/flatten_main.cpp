@@ -27,8 +27,8 @@ int main(int argc, char **argv) {
         std::printf("{\"name\": \"%s\", \"parent\": %d, \"type\": %d, \"idx_q\": %d, \"idx_v\": %d, \"placement\": [",
                     m.joint_names[j].c_str(), m.parent[j], m.jtype[j], m.idx_q[j], m.idx_v[j]);
         for (int k = 0; k < 12; ++k) std::printf("%s%.17g", k ? ", " : "", m.placement[j][k]);
-        std::printf("], \"axis\": [%.17g, %.17g, %.17g]}%s\n", m.axis[j][0], m.axis[j][1], m.axis[j][2],
-                    j + 1 < m.njoints() ? "," : "");
+        std::printf("], \"axis\": [%.17g, %.17g, %.17g], \"mass\": %.17g, \"com\": [%.17g, %.17g, %.17g]}%s\n", m.axis[j][0],
+                    m.axis[j][1], m.axis[j][2], m.mass[j], m.com[j][0], m.com[j][1], m.com[j][2], j + 1 < m.njoints() ? "," : "");
     }
     std::printf("],\n\"frames\": [\n");
     for (int i = 0; i < m.nframes(); ++i) {

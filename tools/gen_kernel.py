@@ -24,7 +24,8 @@ data.cpp:25-58, frame.hpp:37-62,152-182) for a FIXED tree and FIXED frame-task l
 
 The emitted struct is consumed by dls_spec.cuh (thread-per-problem persistent kernel with lane refill) and -- being
 __host__ __device__ -- by the CPU unit-test harness.  Supported: free-flyer or fixed base; RX/RY/RZ/unaligned
-revolute and prismatic joints; FrameTask (Position / Orientation / Full) with the `universe` reference frame.
+revolute, continuous and prismatic joints; FrameTask (Position / Orientation / Full, any reference frame), AlignAxisTask,
+PostureTask and CentreOfMassTask (spec kind "com"; the model JSON then carries each joint's "mass" and "com").
 Anything else runs on the generic kernel.
 """
 import json
@@ -185,6 +186,15 @@ class Generator:
                 row += nj
                 toff += nj
                 continue
+            if kind == "com":  # CentreOfMassTask (centre_of_mass.hpp:14-52): 3 rows, target = the centre of mass in `reference`
+                ref = self.frames[t.get("reference", "universe")]
+                self.tasks.append(dict(frame=ref, kind=kind, ktype=0, dim=3, row=row, toff=toff, tsize=3, chain=self.com_joints(),
+                                       name="com", ref=ref, ref_name=t.get("reference", "universe"), priority=int(t.get("priority", 0))))
+                if int(t.get("priority", 0)) == 0:
+                    self.rows_p0 += 3
+                row += 3
+                toff += 3
+                continue
             f = self.frames[t["frame"]]
             if kind == "frame":
                 ktype = {"position": POSITION, "orientation": ORIENTATION, "full": FULL}[t["type"]]
@@ -210,6 +220,12 @@ class Generator:
                 self.rows_p0 += dim
             row += dim
             toff += tsize
+        if any(t["kind"] == "com" for t in self.tasks):
+            # a com task's columns are not chain-local (every joint that carries mass has one) and its role does its own full
+            # FK: these options assume chain-local columns, one role per limb or were never tested with it
+            for opt in ("arrow_solve", "mirror", "fold_task", "tmem_j", "uniform_solve", "parallel_solve", "presolve", "interleave"):
+                if spec.get(opt) or (opt == "fold_task" and spec.get(opt) is not None):
+                    raise ValueError("spec option %r does not support a centre-of-mass task" % opt)
         self.rows = row
         self.tsz = toff
         self.slots = {}  # (row, col) -> slot index
@@ -231,6 +247,29 @@ class Generator:
         if key not in self.slots:
             self.slots[key] = len(self.slots)
         return self.slots[key]
+
+    # ---- centre of mass ----
+    def com_masses(self):
+        """Subtree masses of every joint (Pinocchio's data.mass[j]), summed children before parents in the order
+        iko_center_of_mass adds them, and the total mass M (the bodies of `universe` itself do not count)."""
+        if any("mass" not in jt or "com" not in jt for jt in self.joints):
+            raise ValueError("a centre-of-mass task needs the per-joint mass and com in the model JSON")
+        ms = [0.0] + [float(jt["mass"]) for jt in self.joints[1:]]
+        M = 0.0
+        for j in range(len(self.joints) - 1, 0, -1):
+            par = self.joints[j]["parent"]
+            if par > 0:
+                ms[par] += ms[j]
+            else:
+                M += ms[j]
+        if not M > 0:
+            raise ValueError("a centre-of-mass task needs a model that carries mass")
+        return ms, M
+
+    def com_joints(self):
+        """joints whose subtree carries mass: the only ones with centre-of-mass Jacobian columns"""
+        ms, _ = self.com_masses()
+        return [j for j in range(1, len(self.joints)) if ms[j] > 0]
 
     # ---- FK of one joint (memoised) ----
     def fk_joint(self, E, j, world):
@@ -434,6 +473,8 @@ class Generator:
             return self.gen_align_task(E, ti, world)
         if self.tasks[ti]["kind"] == "posture":
             return self.gen_posture_task(E, ti)
+        if self.tasks[ti]["kind"] == "com":
+            return self.gen_com_task(E, ti, world)
         if True:
             task = self.tasks[ti]
             f = task["frame"]
@@ -562,6 +603,67 @@ class Generator:
         for i in range(nj):
             E.raw("sE.set(%d, c.weight[%d] * ((q[%d] - tg[%d]) * c.mask[%d]));" % (row + i, row + i, self.nq - nj + i, toff + i, row + i))
             E.raw("sJ.set(%d, c.weight[%d]);  // J[%d][%d]" % (self.slot(row + i, self.nv - nj + i), row + i, row + i, self.nv - nj + i))
+
+    def gen_com_task(self, E, ti, world):
+        """CentreOfMassTask (centre_of_mass.hpp:24-38 with pinocchio::jacobianCenterOfMass, as dls_coop.cuh phases 1b-3 and
+        iko_center_of_mass compute it): with c_j = sum over the subtree of joint j of m_k (R_k com_k + p_k) and M the total mass,
+        e = w o (R_r^T (c / M - p_r) - target) and J = w o R_r^T Jcom, where the column of a coordinate of joint j is
+        share_j v: v = the axis for a prismatic coordinate, axis x (c_j / m_sub(j) - p_j) for a rotation, share_j = m_sub(j) / M.
+        Subtree masses and shares are constants (folded as share_j (c_j / m_sub(j) - p_j) = c_j / M - share_j p_j); the
+        reference frame is not differentiated.  Joints whose subtree carries no mass get no columns."""
+        task = self.tasks[ti]
+        row, toff = task["row"], task["toff"]
+        E.comment("==== task %d: centre of mass, reference %s ====" % (ti, task["ref_name"]))
+        ms, M = self.com_masses()
+        used = task["chain"]
+        for j in used:
+            self.fk_joint(E, j, world)
+        # first moments of the bodies of every joint, then ONE backward sweep over the tree
+        own = {}
+        for j in used:
+            m, cj, w = float(self.joints[j]["mass"]), [float(x) for x in self.joints[j]["com"]], world[j]
+            if m > 0:
+                cw = [sop(E, [(w["R"][3 * i + k], cj[k]) for k in range(3)], "cw", w["p"][i]) for i in range(3)]
+                own[j] = [sop(E, [(m, cw[i])], "mc") for i in range(3)]
+            else:
+                own[j] = [0.0, 0.0, 0.0]
+        csub = {}
+        for j in sorted(used, reverse=True):   # children (higher indices) first; a parent adds them highest index first
+            kids = sorted((k for k in used if self.joints[k]["parent"] == j), reverse=True)
+            csub[j] = [sop(E, [(1.0, own[j][i])] + [(1.0, csub[k][i]) for k in kids], "cs") for i in range(3)]
+        roots = sorted((k for k in used if self.joints[k]["parent"] == 0), reverse=True)
+        com = [E.var("(%s) / %s" % (lit(sop(E, [(1.0, csub[k][i]) for k in roots], "ct")), lit(M)), "cm") for i in range(3)]
+        if self.is_universe(task["ref"]):
+            Rr, lc = None, com
+        else:
+            Rr, pr = self.frame_world(E, task["ref"], world, "r")
+            d = sub3(E, com, pr, "cd")
+            lc = [sop(E, [(Rr[3 * k + i], d[k]) for k in range(3)], "cl") for i in range(3)]
+        for i in range(3):
+            E.raw("sE.set(%d, c.weight[%d] * (%s - tg[%d]));" % (row + i, row + i, lit(lc[i]), toff + i))
+
+        def column(col, vel):
+            for i in range(3):
+                val = vel[i] if Rr is None else sop(E, [(Rr[3 * k + i], vel[k]) for k in range(3)], "jc")
+                if is_const(val) and val == 0:
+                    continue   # structurally zero: no slot
+                E.raw("sJ.set(%d, c.weight[%d] * %s);  // J[%d][%d]" % (self.slot(row + i, col), row + i, lit(val), row + i, col))
+
+        for j in used:
+            jt, w = self.joints[j], world[j]
+            iv, share = jt["idx_v"], ms[j] / M
+            dsh = [sop(E, [(csub[j][i], 1.0 / M), (w["p"][i], share, -1)], "dc") for i in range(3)]
+            if jt["type"] == J_FF:   # LOCAL columns: linear along R e_k, angular about R e_k through p
+                for k in range(3):
+                    ek = [w["R"][k], w["R"][3 + k], w["R"][6 + k]]
+                    column(iv + k, [sop(E, [(share, ek[i])], "cv") for i in range(3)])
+                for k in range(3):
+                    ek = [w["R"][k], w["R"][3 + k], w["R"][6 + k]]
+                    column(iv + 3 + k, [_cross_comp(E, ek, dsh, i, "cv") for i in range(3)])
+            elif jt["type"] in J_REV:
+                column(iv, [_cross_comp(E, w["z"], dsh, i, "cv") for i in range(3)])
+            else:   # prismatic
+                column(iv, [sop(E, [(share, w["z"][i])], "cv") for i in range(3)])
 
     def gen_align_task(self, E, ti, world):
         """AlignAxisTask (frame.hpp:246-299): e = 1 - r . t^,  J = -(r x t^)^T R_rMf Jf_LOCAL.bottomRows(3), with r the
@@ -1815,6 +1917,7 @@ class Generator:
         for k, (g, ev) in enumerate(zip(groups, evs)):
             names = ", ".join("%s %s" % (self.tasks[t]["name"], ("align-" + "xyz"[self.tasks[t]["ktype"]]) if self.tasks[t]["kind"] == "align"
                                          else "" if self.tasks[t]["kind"] == "posture"
+                                         else "(reference %s)" % self.tasks[t]["ref_name"] if self.tasks[t]["kind"] == "com"
                                          else ["Position", "Orientation", "Full"][self.tasks[t]["ktype"]]) for t in g)
             out.append("    // ---- role %d: %s ----" % (k, names))
             out.append("    // copy this role's target poses into the strip sT")
@@ -2121,7 +2224,7 @@ class Generator:
                    ", ".join(str(t["ktype"]) for t in self.tasks))
         out.append("    // task kind (0 frame, 1 align-axis, 2 posture; sig_task_type is the axis / the number of coordinates for those)")
         out.append("    static const int *sig_task_kind() { static const int v[] = {%s}; return v; }" %
-                   ", ".join({"frame": "0", "align": "1", "posture": "2"}[t["kind"]] for t in self.tasks))
+                   ", ".join({"frame": "0", "align": "1", "posture": "2", "com": "3"}[t["kind"]] for t in self.tasks))
         out.append("    static const int *sig_task_ref_joint() { static const int v[] = {%s}; return v; }" %
                    ", ".join(str(t["ref"]["parent"]) for t in self.tasks))
         rpl = []
@@ -2138,6 +2241,12 @@ class Generator:
             fpl.extend(t["frame"]["placement"])
         out.append("    static const double *sig_task_placement() { static const double v[] = {%s}; return v; }" %
                    ", ".join(repr(float(x)) for x in fpl))
+        if any(t["kind"] == "com" for t in self.tasks):
+            # the masses and centres of mass folded into the com task's code: a problem whose model carries other inertias
+            # must not match (dls_spec.cuh spec_has_inertia); emitted only for specs with a com task
+            out.append("    // per joint: mass, then its centre of mass in the joint frame (3) -- the com task's folded constants")
+            out.append("    static const double *sig_inertia() { static const double v[] = {%s}; return v; }" %
+                       ", ".join(repr(float(x)) for jt in self.joints for x in [jt["mass"]] + list(jt["com"])))
         out.append("};")
         out.append("}  // namespace ikb")
         # The Jacobian strip has a type of its own (SJ): the kernel may keep it in tensor memory (TStrip, tmem_scratch.cuh)
