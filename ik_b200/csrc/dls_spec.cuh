@@ -74,6 +74,58 @@ struct DynSmemOptIn {
 #define IKB_TMEM_J 1
 #endif
 template <class Spec, typename T> constexpr bool spec_tmem_j() { return IKB_TMEM_J && IKB_TMEM_Q && Spec::ARROW && Spec::TMEMJ && sizeof(T) == 8 && Spec::NQL <= 16; }
+// Spec::qstage_l(role) (TMEMJ specs only): first of NQ factor-strip slots where a converged slot's next configuration is
+// staged for that role; does every role of the spec have such a home?
+template <class Spec, class = void> struct spec_qstage_l { static constexpr bool value = false; };
+template <class Spec> struct spec_qstage_l<Spec, std::void_t<decltype(Spec::qstage_l(0))>> {
+    static constexpr bool all(int r) { return r >= Spec::NWARPS || (Spec::qstage_l(r) >= 0 && all(r + 1)); }
+    static constexpr bool value = all(0);
+};
+
+// IKB_TRIP_PROFILE=1 (tools/trip_profile.py; never in the library): the merged launch of a TMEMJ body adds up, per warp role,
+// the clock64() cycles of each segment of a trip into ikb_trip_cycles (kTripSegs counters per role, then the trip count)
+#ifndef IKB_TRIP_PROFILE
+#define IKB_TRIP_PROFILE 0
+#endif
+enum TripSeg { kTripTopBarrier, kTripTmemFetch, kTripEvaluate, kTripPhase1, kTripStopTest, kTripPhase23, kTripBarrier2,
+               kTripStep, kTripResults, kTripRefill, kTripPark, kTripSegs };
+#if IKB_TRIP_PROFILE
+static __device__ unsigned long long ikb_trip_cycles[4 * (kTripSegs + 1)];
+#endif
+struct TripClock {
+#if IKB_TRIP_PROFILE
+    long long t = 0, acc[kTripSegs] = {}, trips = 0;
+    __device__ void start() { t = clock64(); }
+    __device__ void trip() { ++trips; }
+    __device__ void mark(int seg) {
+        const long long now = clock64();
+        acc[seg] += now - t;
+        t = now;
+    }
+    // the results / refill split of the end of a trip: lanes run it divergently, so the warp's split point is the first
+    // lane's `at` (0: this lane did not finish)
+    __device__ void split(long long at) {
+        unsigned d = at ? (unsigned)(at - t) : 0xffffffffu;
+        d = __reduce_min_sync(0xffffffffu, d);
+        if (d != 0xffffffffu) {
+            acc[kTripResults] += d;
+            t += d;
+        }
+        mark(kTripRefill);
+    }
+    __device__ void flush(int role) {
+        if ((threadIdx.x & 31) != 0) return;
+        for (int k = 0; k < kTripSegs; ++k) atomicAdd(&ikb_trip_cycles[role * (kTripSegs + 1) + k], (unsigned long long)acc[k]);
+        atomicAdd(&ikb_trip_cycles[role * (kTripSegs + 1) + kTripSegs], (unsigned long long)trips);
+    }
+#else
+    __device__ void start() {}
+    __device__ void trip() {}
+    __device__ void mark(int) {}
+    __device__ void split(long long) {}
+    __device__ void flush(int) {}
+#endif
+};
 // tensor-memory columns of a warp role: 32 for the parked configuration + two per Jacobian slot of the role
 template <class Spec, typename T> constexpr int spec_tmem_width(int role) { return 32 + (spec_tmem_j<Spec, T>() ? 2 * Spec::j_count(role) : 0); }
 // columns in use in lane quarter `quarter` when the CTA has `nwarps` warps (warp w: quarter w % 4, role w % NWARPS)
@@ -134,9 +186,34 @@ __global__ void __launch_bounds__(GROUPS *Spec::NWARPS * 32, MINB)
     // of the staged configuration with shared-memory loads; the global round trip that used to end every trip of every
     // role (3-4 of a group's 32 slots refill per trip) is gone from the critical roles' path.  Slots that finish
     // without converging, carried stragglers and the TAIL launch take the direct path (load_problem).
-    constexpr bool kPrefetch = Spec::ARROW && NW > 1 && !kTmemJ && !Spec::CAPSOLO && Spec::QSTAGE >= 0 && IKB_PREFETCH;
-    const S sQ{sm + (kPrefetch ? Spec::QSTAGE : 0) * SLOTS};
+    // TMEMJ bodies (the Jacobian rows in tensor memory) stage the configuration in the factor strip instead, one copy per
+    // role in the role's OWN published contributions (Spec::qstage_l): they are dead from the second barrier on, and the
+    // next store into them is the role's own phase 1, after its loads in program order -- the roles run unordered from the
+    // top barrier to the one inside psolve(), so a slot another role stores first would race with the loads.  The copies
+    // are issued behind the second barrier and waited for at the end of the trip (kStager below); every role picks its
+    // coordinates up behind the barrier at the top of the next trip.
+    constexpr bool kPrefetch = Spec::ARROW && NW > 1 && !Spec::CAPSOLO && (kTmemJ ? spec_qstage_l<Spec>::value : Spec::QSTAGE >= 0) && IKB_PREFETCH;
+    auto stage_at = [&](int r) -> T * {                     // the staged configuration role r reads
+        if constexpr (kTmemJ && kPrefetch) return sm + (kJS + Spec::qstage_l(r)) * SLOTS;
+        else return sm + (kPrefetch ? Spec::QSTAGE : 0) * SLOTS;
+    };
     constexpr long long kStagedBit = 1LL << 62;             // in *sNext: the ticket's problem is already staged
+    bool staged = false;    // (TMEMJ) this slot's next problem waits in the staging slots for the top of the next trip
+    // TMEMJ: the SOLVER role carries the longer trip (stop test, free-flyer step, mailbox), so the copies are issued by
+    // another role -- right after the second barrier, when the ticket is visible and the contributions are dead -- which
+    // waits for them at the end of its trip, in the slack it used to spend at the barrier at the top of the loop
+    constexpr int kStager = kTmemJ ? (Spec::SOLVER + 1) % NW : Spec::SOLVER;
+    auto stage = [&](long long idx) {
+        const ProblemIO<T> io = problem_io<SEG>(a, idx);
+#pragma unroll
+        for (int r = 0; r < NW; ++r) Spec::load_targets(r, io.targets, io.tg_es, sT);
+#pragma unroll
+        for (int r = 0; r < (kTmemJ ? NW : 1); ++r) {
+            const S sQ{stage_at(r)};
+#pragma unroll
+            for (int k = 0; k < NQ; ++k) sQ.copy_in(k, io.q0 + k * io.q0_es);
+        }
+    };
 
     auto group_sync = [&]() {
         if constexpr (NW > 1)
@@ -249,8 +326,24 @@ __global__ void __launch_bounds__(GROUPS *Spec::NWARPS * 32, MINB)
             return __any_sync(0xffffffffu, have) != 0;
         }
     };
+    constexpr bool kTripProf = IKB_TRIP_PROFILE && kTmemJ && SEG;
+    TripClock tc;
+    auto tmark = [&](int seg) {
+        if constexpr (kTripProf) tc.mark(seg);
+    };
+    if constexpr (kTripProf) tc.start();
     while (any_left()) {
+        tmark(kTripTopBarrier);
+        if constexpr (kTripProf) tc.trip();
         if constexpr (kTmemQ) tmem_fetch(tmem_q, q);        // (all lanes: the transfer is warp-wide)
+        if constexpr (kPrefetch && kTmemJ) {
+            if (__any_sync(0xffffffffu, staged)) {          // landed: the staging role waited before the barrier
+                if (staged) Spec::load_q(role, stage_at(role), (long long)SLOTS, q);
+                tmem_park(tmem_q, q);                       // (warp-wide) the step fetches q from tensor memory again
+            }
+            staged = false;
+        }
+        tmark(kTripTmemFetch);
         if constexpr (Spec::QCOMMON) {
             if (have && refetch) Spec::fetch_common(role, sL, q);   // the coordinates the solver role stepped for everybody
             refetch = false;
@@ -260,6 +353,7 @@ __global__ void __launch_bounds__(GROUPS *Spec::NWARPS * 32, MINB)
             // (on stale or arbitrary inputs; nobody reads what they produce)
             Spec::evaluate(role, q, sT, c, sJ, sE);
             sJ.flush();
+            tmark(kTripEvaluate);
         } else if (have) {
             Spec::evaluate(role, q, sT, c, sJ, sE);         // data.cpp:25-58, this role's tasks
             // The solver role's own tasks are the cheap ones: while the others still evaluate, it factorises the leading
@@ -291,11 +385,7 @@ __global__ void __launch_bounds__(GROUPS *Spec::NWARPS * 32, MINB)
                 long long nb = (long long)atomicAdd(a.ticket, 1ULL);
                 if constexpr (kPrefetch) {
                     if (res < a.tolerance && !a.resume && nb >= ncarry && nb - ncarry < a.B) {   // converged here, a fresh problem next
-                        const ProblemIO<T> io = problem_io<SEG>(a, nb - ncarry);
-#pragma unroll
-                        for (int r = 0; r < NW; ++r) Spec::load_targets(r, io.targets, io.tg_es, sT);
-#pragma unroll
-                        for (int k = 0; k < NQ; ++k) sQ.copy_in(k, io.q0 + k * io.q0_es);
+                        if constexpr (!kTmemJ) stage(nb - ncarry);
                         nb |= kStagedBit;
                     }
                 }
@@ -310,10 +400,29 @@ __global__ void __launch_bounds__(GROUPS *Spec::NWARPS * 32, MINB)
             // Bordered-block-diagonal step (gen_solve_arrow): phase 1 on the role's own rows, ONE barrier, the stop test
             // (solver role, all of e visible), the small shared-column system in every role, y for the role's own rows.
             T y[Spec::MY];
-            Spec::psolve(role, sJ, sL, sE, a.damping2, y, group_sync, stop_test);
-            if constexpr (kPrefetch)
+            if constexpr (kTripProf) {
+                auto sync1 = [&]() {
+                    group_sync();
+                    tmark(kTripPhase1);
+                };
+                auto hook = [&]() {
+                    stop_test();
+                    tmark(kTripStopTest);
+                };
+                Spec::psolve(role, sJ, sL, sE, a.damping2, y, sync1, hook);
+                tmark(kTripPhase23);
+            } else {
+                Spec::psolve(role, sJ, sL, sE, a.damping2, y, group_sync, stop_test);
+            }
+            if constexpr (kPrefetch && !kTmemJ)
                 if (role == Spec::SOLVER) strip_copies_wait();   // the staged problems have landed before the others look
             if constexpr (!Spec::CAPSOLO) group_sync();     // s and ||e||^2 visible (y is role-private)
+            tmark(kTripBarrier2);
+            if constexpr (kPrefetch && kTmemJ)
+                if (role == kStager && have && abs_(*sRes) < a.tolerance) {   // converged: *sNext is this trip's ticket
+                    const long long nb = *sNext;
+                    if (nb & kStagedBit) stage((nb & ~kStagedBit) - ncarry);
+                }
             if constexpr (kTmemQ) tmem_fetch(tmem_q, q);    // back for the step (a non-solver role's copy of the common
                                                             // coordinates is stale here: it neither steps nor stores them)
             if constexpr (kTmemJ) {
@@ -327,6 +436,7 @@ __global__ void __launch_bounds__(GROUPS *Spec::NWARPS * 32, MINB)
 #pragma unroll
                 for (int k = 0; k < Spec::NQL; ++k) q[k] = go ? qn[k] : q[k];
                 if (go) refetch = true;
+                tmark(kTripStep);
             } else if (have && !(abs_(*sRes) < a.tolerance)) {     // dls.cpp:52,61-71
                 if constexpr (Spec::MY != M) Spec::step_role(role, sJ, sL, q, a.step_length, c, y);   // y in the role's registers
                 else Spec::step_role(role, sJ, sL, q, a.step_length, c);
@@ -358,6 +468,7 @@ __global__ void __launch_bounds__(GROUPS *Spec::NWARPS * 32, MINB)
         }
         // (ARROW: nothing a role writes from here to the CTA-wide barrier at the top of the loop is read by another role)
         if constexpr (!Spec::ARROW) group_sync();           // ||e||^2, dq (and the next ticket) visible; J, e, factor dead
+        [[maybe_unused]] long long tp_refill = 0;   // (IKB_TRIP_PROFILE)
         if (have) {
             const T sres = *sRes;
             const bool suspend = sres < T(0);               // bulk launch: hand the straggler to the tail launch
@@ -394,15 +505,17 @@ __global__ void __launch_bounds__(GROUPS *Spec::NWARPS * 32, MINB)
                         if (io.resid) *io.resid = res;
                     }
                 }
+                if constexpr (kTripProf) tp_refill = clock64();
                 b = *sNext;
                 if constexpr (kPrefetch) {
-                    if (b & kStagedBit) {                    // staged by the SOLVER role during this trip
+                    if (b & kStagedBit) {                    // staged during this trip
                         b = (b & ~kStagedBit) - ncarry;
                         it = 0;
                         refetch = false;
                         carried = false;
                         have = true;
-                        Spec::load_q(role, sQ.base, (long long)SLOTS, q);
+                        if constexpr (kTmemJ) staged = true;     // (the copies may still be in flight)
+                        else Spec::load_q(role, stage_at(0), (long long)SLOTS, q);
                     } else {
                         load_problem();
                     }
@@ -411,7 +524,15 @@ __global__ void __launch_bounds__(GROUPS *Spec::NWARPS * 32, MINB)
                 }
             }
         }
+        if constexpr (kPrefetch && kTmemJ)
+            if (role == kStager) strip_copies_wait();       // the staged problems land before the barrier at the top
+        if constexpr (kTripProf) tc.split(tp_refill);
         if constexpr (kTmemQ) tmem_park(tmem_q, q);         // stepped, refilled or unchanged: out of the registers again
+        tmark(kTripPark);
+    }
+    if constexpr (kTripProf) {
+        tmark(kTripTopBarrier);
+        tc.flush(role);
     }
     if constexpr (kTmemQ) tmem_release<kTmemCols>(tmem_base, warp);
 }

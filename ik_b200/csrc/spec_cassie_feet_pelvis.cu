@@ -150,3 +150,13 @@ int l32(const SpecHostConsts &hc, const SolveArgs<float> &a, int v, long long n,
 }  // namespace
 extern const SpecializedKernel kSpecCassieFeetPelvis = {S3::name(), spec_matches<S3>, l64, l32, spec_near_miss<S3>};
 }  // namespace ikb
+
+#if IKB_TRIP_PROFILE
+// tools/trip_profile.py: copy out (and zero) the trip-segment counters of the merged fold launches (dls_spec.cuh, TripClock)
+extern "C" int ikb_trip_profile(unsigned long long *out, int n) {
+    static const unsigned long long zero[4 * (ikb::kTripSegs + 1)] = {};
+    if (n * 8 > (int)sizeof(zero)) return 1;
+    if (out && cudaMemcpyFromSymbol(out, ikb::ikb_trip_cycles, n * 8) != cudaSuccess) return 1;
+    return cudaMemcpyToSymbol(ikb::ikb_trip_cycles, zero, sizeof(zero)) == cudaSuccess ? 0 : 1;
+}
+#endif

@@ -1275,6 +1275,40 @@ class Generator:
                 name[k0 + i] = "%s[%d]" % (nm, i)
         return head + [pat.sub(lambda mt: name[int(mt.group(1))], ln) for ln in lines]
 
+    def factor_stage_slots(self):
+        """Spec "tmem_j": per warp role, the first of NQ consecutive factor-strip slots where the kernel may stage a converged
+        slot's NEXT configuration for that role (dls_spec.cuh, kPrefetch), or None if some role has no such run.  The kernel
+        copies behind the second barrier, and the role reads its slots behind the barrier at the top of the next trip.
+          * Under TMEMJ every lane runs phase 2, phase 3 and step_role warp-wide, also the lanes whose problem converged, so
+            no slot they store qualifies: not e (read by phase 3), not s, not the mailbox or the common coordinates (stored
+            by step_role), not a factor (its slots carry y where y is not in registers).
+          * Between the top barrier and the next barrier (inside psolve()) the roles run unordered, so the next store into
+            a role's staging slots must come from that role itself, after its loads in program order.  That leaves the role's
+            OWN published contributions: its phase 1 stores them, phase 2 reads them before the second barrier, and no
+            other role stores them.  (The fold task's contributions are stored by every role's evaluate: never used.)"""
+        A = self.arrow
+        if self.spec.get("arrow_cap_solo"):
+            return None
+        per = A["ks"] * (A["ks"] + 1) // 2 + A["ks"]
+        dead = set(range(self.rows)) | set(range(A["soff"], A["soff"] + A["ks"]))
+        if self.arrow_mail:
+            dead |= set(x for v in self.arrow_mail.values() for x in v)
+        if self.arrow_qc is not None:
+            dead |= set(range(self.arrow_qc, self.arrow_qc + A["ncq"]))
+        for base in A["facb"].values():
+            dead |= set(range(base, base + A["my"] * (A["my"] + 1) // 2))
+        out = []
+        for k in sorted(A["pub"]):
+            if k == A["fold"]:
+                continue
+            kind, where = A["pub"][k]
+            ok = set(range(where, where + per)) - dead if kind == "L" else set()
+            k0 = next((k0 for k0 in sorted(ok) if all(k0 + i in ok for i in range(self.nq))), None)
+            if k0 is None:
+                return None
+            out.append(k0)
+        return out
+
     def gen_solve_arrow(self, groups, solver, fold=None):
         """Spec "arrow_solve": the step WITHOUT the dense M x M factorisation, for task sets whose Jacobian is "bordered block
         diagonal": a few columns (the free-flyer; joints that several limbs' tasks share) are touched by several warp
@@ -1596,7 +1630,7 @@ class Generator:
         for i in range(ks - 1, -1, -1):
             Cc.append(ind + "s[%d] = cz%d * ci%d%s;" % (i, i, i, "".join(" - cl%d_%d * s[%d]" % (j, i, j) for j in range(i + 1, ks))))
         self.arrow = dict(shared=shared, spos=spos, soff=SOFF, ks=ks, nfact=nfact, fma=nf, mirror_of=mirror_of,
-                          pub=pub, facb=facb, fac_regs=fac_regs, y_regs=y_regs, nfac=mmax * (mmax + 1) // 2 if fac_regs else 1, my=mmax)
+                          pub=pub, facb=facb, fac_regs=fac_regs, y_regs=y_regs, ncq=ncq, fold=fold, nfac=mmax * (mmax + 1) // 2 if fac_regs else 1, my=mmax)
         self.rhs_off = 0
         return locals_, Cc, finishes
 
@@ -1908,6 +1942,12 @@ class Generator:
                     break
         out.append("    // QSTAGE: first of NQ Jacobian slots where the kernel may stage the next problem's configuration (-1: none)")
         out.append("    static constexpr int QSTAGE = %d;" % qstage)
+        if tmemj:
+            st = self.factor_stage_slots()
+            out.append("    // qstage_l: first of NQ factor-strip slots where the kernel may stage the next problem's configuration for a role,")
+            out.append("    // in the role's own published contributions (-1: no staging)")
+            out.append("    static constexpr int qstage_l(int role) { return %s; }" %
+                       " : ".join(["role == %d ? %d" % (r, k0) for r, k0 in enumerate(st or [])] + ["-1"]))
         out.append("    // CAPSOLO: psolve() ends behind a barrier of its own (the shared-column system is solved by the SOLVER role alone)")
         out.append("    static constexpr bool CAPSOLO = %s;" % ("true" if arrow and self.spec.get("arrow_cap_solo") else "false"))
         out.append("    // PRE: leading rows whose P x P factor block the SOLVER role computes in presolve(), before the first barrier;")
