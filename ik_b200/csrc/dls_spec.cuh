@@ -550,6 +550,29 @@ inline bool same_values(const double *a, const double *b, int n) {  // value equ
 template <class Spec, class = void> struct spec_has_inertia : std::false_type {};
 template <class Spec> struct spec_has_inertia<Spec, std::void_t<decltype(Spec::sig_inertia())>> : std::true_type {};
 
+// Specs generated with FrameConstraints project every step onto their null space and carry the constraint list as
+// Spec::sig_con_type() etc. (NCONS entries in stacked order); the other generated headers have no such member.
+template <class Spec, class = void> struct spec_has_constraints : std::false_type {};
+template <class Spec> struct spec_has_constraints<Spec, std::void_t<decltype(Spec::sig_con_type())>> : std::true_type {};
+
+// Does the problem's constraint list have the Spec's structure: count, order, type, frame and reference joints?
+// (A Spec without constraints: only an empty list.)
+template <class Spec> bool spec_constraint_structure(const HostProblem &hp) {
+    if constexpr (spec_has_constraints<Spec>::value) {
+        if ((int)hp.constraints.size() != Spec::NCONS) return false;
+        const HostModel &m = hp.model;
+        for (int k = 0; k < Spec::NCONS; ++k) {
+            const HostConstraint &hc = hp.constraints[k];
+            if (hc.type != Spec::sig_con_type()[k] || m.frame_parent[hc.frame] != Spec::sig_con_joint()[k] ||
+                m.frame_parent[hc.ref] != Spec::sig_con_ref_joint()[k])
+                return false;
+        }
+        return true;
+    } else {
+        return hp.constraints.empty();
+    }
+}
+
 // generator task kind code (sig_task_kind) -> HostTask::kind
 constexpr int kSpecTaskKinds[4] = {IKB_TASK_FRAME, IKB_TASK_ALIGN_AXIS, IKB_TASK_POSTURE, IKB_TASK_COM};
 
@@ -588,6 +611,15 @@ template <class Spec> bool spec_matches(const HostProblem &hp) {
         if (m.frame_parent[ht.frame] != Spec::sig_task_joint()[t]) return false;
         if (!same_values(m.frame_placement[ht.frame].data(), Spec::sig_task_placement() + 12 * t, 12)) return false;
     }
+    // the constraints, in the order Jc stacks them, with the frame placements their code was generated for
+    if (!spec_constraint_structure<Spec>(hp)) return false;
+    if constexpr (spec_has_constraints<Spec>::value) {
+        for (int k = 0; k < Spec::NCONS; ++k) {
+            const HostConstraint &hc = hp.constraints[k];
+            if (!same_values(m.frame_placement[hc.frame].data(), Spec::sig_con_placement() + 12 * k, 12)) return false;
+            if (!same_values(m.frame_placement[hc.ref].data(), Spec::sig_con_ref_placement() + 12 * k, 12)) return false;
+        }
+    }
     return true;
 }
 
@@ -598,7 +630,7 @@ template <class Spec> bool spec_near_miss(const HostProblem &hp, std::string *wh
     const HostModel &m = hp.model;
     if (m.njoints() != Spec::NJOINTS || m.nq != Spec::NQ || m.nv != Spec::NV) return false;
     if ((int)hp.tasks.size() != Spec::NTASKS || hp.rows() != Spec::M || hp.e_size(0) != Spec::M0) return false;
-    if (!hp.constraints.empty()) return false;
+    if (!spec_constraint_structure<Spec>(hp)) return false;
     const int *par = Spec::sig_parent(), *typ = Spec::sig_type();
     for (int j = 0; j < Spec::NJOINTS; ++j)
         if (m.parent[j] != par[j] || m.jtype[j] != typ[j]) return false;
@@ -630,6 +662,13 @@ template <class Spec> bool spec_near_miss(const HostProblem &hp, std::string *wh
         if (ht.kind == IKB_TASK_POSTURE) continue;
         scan(m.frame_placement[ht.ref].data(), Spec::sig_task_ref_placement() + 12 * t, 12, "reference frame of task", t, m.frame_names[ht.ref].c_str());
         scan(m.frame_placement[ht.frame].data(), Spec::sig_task_placement() + 12 * t, 12, "frame of task", t, m.frame_names[ht.frame].c_str());
+    }
+    if constexpr (spec_has_constraints<Spec>::value) {
+        for (int k = 0; k < Spec::NCONS; ++k) {
+            const HostConstraint &hc = hp.constraints[k];
+            scan(m.frame_placement[hc.frame].data(), Spec::sig_con_placement() + 12 * k, 12, "frame of constraint", k, m.frame_names[hc.frame].c_str());
+            scan(m.frame_placement[hc.ref].data(), Spec::sig_con_ref_placement() + 12 * k, 12, "reference frame of constraint", k, m.frame_names[hc.ref].c_str());
+        }
     }
     if (!(worst > 0)) return false;   // equal values: not a miss at all (IKB_FORCE_GENERIC, task order, ...)
     if (why) {

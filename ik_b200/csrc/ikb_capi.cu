@@ -102,9 +102,9 @@ int launch_fk(const ikb_problem *p, int64_t B, const void *q, int64_t es, int64_
 }
 
 // The specialised bodies lay targets out in stacked order, the ABI in insertion order: only problems whose tasks
-// were added in non-decreasing priority (stacked order == insertion order) can take the fast path.
+// were added in non-decreasing priority (stacked order == insertion order) can take the fast path.  A problem with
+// FrameConstraints matches only a specialisation generated for the same constraint list (spec_matches).
 const SpecializedKernel *select_specialized(const HostProblem &hp) {
-    if (!hp.constraints.empty()) return nullptr;  // the null-space projection lives in the table-driven kernel
     for (size_t i = 1; i < hp.tasks.size(); ++i)
         if (hp.tasks[i].priority < hp.tasks[i - 1].priority) return nullptr;
     return find_specialized(hp);
@@ -549,7 +549,7 @@ int ikb_problem_finalize(ikb_problem *p, int device) {
     if (!p->spec) {
         const char *forced = std::getenv("IKB_FORCE_GENERIC");
         std::string why;
-        if (!(forced && forced[0] == '1') && hp.constraints.empty() && find_near_miss(hp, &why)) {
+        if (!(forced && forced[0] == '1') && find_near_miss(hp, &why)) {
             p->status = why;
             const char *quiet = std::getenv("IKB_QUIET");
             static std::atomic<bool> warned{false};

@@ -10,8 +10,8 @@ translation (ik_ros/src/cassie.cpp:95-96).  The initial guess is the SRDF standi
 """
 import numpy as np
 
-from .api import (AlignAxisTask, AlignAxisType, CentreOfMassTask, FrameTask, InverseKinematicsProblem, KinematicType,
-                  Model, PostureTask)
+from .api import (AlignAxisTask, AlignAxisType, CentreOfMassTask, FrameConstraint, FrameTask, InverseKinematicsProblem,
+                  KinematicType, Model, PostureTask)
 
 # cassie-description/srdf/cassie.srdf:22-39 (group_state "default"), in model joint order
 CASSIE_STANDING = [0.0045, 0.0, 0.4973, -1.1997, 0.0, 1.4267, 0.0, -1.5968,
@@ -166,6 +166,47 @@ def cassie_com_problem(model=None, reference="universe"):
     pb.add_frame_task("fr", FrameTask(model, "RightFootFront", KinematicType.Position))
     pb.add_frame_task("pelvis", FrameTask(model, "pelvis", KinematicType.Orientation))
     return pb
+
+
+def cassie_constraint_problem(model=None, ktype=KinematicType.Position, reference="universe"):
+    """Cassie with a planted foot: pelvis Full and LeftFootFront Position tasks (9 task rows), RightFootFront held in place
+    relative to `reference` by a FrameConstraint of type `ktype` (ik::dls projects every step onto its null space)."""
+    model = model or cassie_model()
+    pb = InverseKinematicsProblem(model, 0)
+    pb.add_frame_task("pelvis", FrameTask(model, "pelvis", KinematicType.Full))
+    pb.add_frame_task("fl", FrameTask(model, "LeftFootFront", KinematicType.Position))
+    pb.add_frame_constraint("fr", FrameConstraint(model, "RightFootFront", ktype, reference))
+    return pb
+
+
+def cassie_stance_problem(model=None, reference="universe"):
+    """Cassie in double stance: a pelvis Full task (6 rows) with both feet pinned relative to `reference` by Full
+    FrameConstraints -- 12 constraint rows, the most a problem may have.  Draw its targets with cassie_stance_targets()."""
+    model = model or cassie_model()
+    pb = InverseKinematicsProblem(model, 0)
+    pb.add_frame_task("pelvis", FrameTask(model, "pelvis", KinematicType.Full))
+    pb.add_frame_constraint("fl", FrameConstraint(model, "LeftFootFront", KinematicType.Full, reference))
+    pb.add_frame_constraint("fr", FrameConstraint(model, "RightFootFront", KinematicType.Full, reference))
+    return pb
+
+
+def cassie_stance_targets(problem, B, seed=12345, b0=0):
+    """Pelvis targets [B, tsz] that the pinned feet of cassie_stance_problem() leave reachable from the standing pose: the
+    standing pelvis placement (identity, at the origin) moved by U[-0.01, 0.01]^3 m and turned by exp3(u), u uniform in
+    [-0.01, 0.01]^3 rad (problem indices b0 .. b0+B-1).  With both feet held, pelvis moves of a few centimetres are mostly
+    out of reach: ik::dls converges on about 80 % of these draws in 60 half steps, on 5 % of +-3 cm / +-0.05 rad ones."""
+    b = np.arange(b0, b0 + B, dtype=np.uint64)
+    tg = np.zeros((B, problem.target_size))
+    off = problem.target_offset(problem.get_frame_task("pelvis"))
+    u = np.stack([-0.01 + 0.02 * uniform01(seed, b, 3 + i) for i in range(3)], axis=1)
+    th = np.maximum(np.linalg.norm(u, axis=1), 1e-300)[:, None, None]
+    K = np.zeros((B, 3, 3))
+    K[:, 0, 1], K[:, 0, 2], K[:, 1, 2] = -u[:, 2], u[:, 1], -u[:, 0]
+    K -= K.transpose(0, 2, 1)
+    R = np.eye(3) + np.sin(th) / th * K + (1 - np.cos(th)) / th ** 2 * (K @ K)
+    tg[:, off:off + 9] = R.reshape(B, 9)
+    tg[:, off + 9:off + 12] = np.stack([-0.01 + 0.02 * uniform01(seed, b, i) for i in range(3)], axis=1)
+    return tg
 
 
 def com_targets(problem, targets, coms, poses=None):

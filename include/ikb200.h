@@ -140,7 +140,9 @@ int ikb_model_set_inertias(ikb_model *m, const double *mass, const double *com);
 /* FrameConstraint (reference frame.hpp:333-465; problem.hpp add_frame_constraint): ik::dls projects its step into the null
  * space of the stacked constraint Jacobian, N = I - Jc.completeOrthogonalDecomposition().pseudoInverse() Jc
  * (dls.cpp:26-34,44-52), i.e. keeps `frame` at rest relative to `ref`.  Returns the constraint index or minus an
- * ikb_status.  At most 4 constraints / 12 rows; problems with constraints run on the table-driven kernel. */
+ * ikb_status.  At most 4 constraints / 12 rows; problems with constraints run on the table-driven kernel unless a loaded
+ * plugin generated for the same constraint list matches (ikb_load_specialisation; same count, order, types, frames,
+ * reference frames and frame placements). */
 int ikb_problem_add_frame_constraint(ikb_problem *p, int frame, int ktype, int ref);
 int ikb_problem_c_size(const ikb_problem *p); /* InverseKinematicsProblem::c_size(), problem.hpp:47-53 */
 int ikb_problem_num_tasks(const ikb_problem *p);

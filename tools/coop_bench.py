@@ -68,15 +68,6 @@ def run(name, make, B, start, solve=None, com=None, legacy_ok=True):
             name, v, pb.kernel_name(), B, ms, conv / ms / 1e3, conv / B, out["iters"].float().mean().item(), note), flush=True)
 
 
-def constraint_pb():
-    m = W.cassie_model()
-    pb = ik.InverseKinematicsProblem(m, 0)
-    pb.add_frame_task("pelvis", ik.FrameTask(m, "pelvis", ik.KinematicType.Full))
-    pb.add_frame_task("fl", ik.FrameTask(m, "LeftFootFront", ik.KinematicType.Position))
-    pb.add_frame_constraint("fr", ik.FrameConstraint(m, "RightFootFront", ik.KinematicType.Position))
-    return pb
-
-
 def com_pb():
     m = W.cassie_model()
     pb = ik.InverseKinematicsProblem(m, 0)
@@ -90,7 +81,7 @@ def com_pb():
 run("cassie feet+pelvis", W.cassie_feet_pelvis_problem, 65536, "standing")
 run("cassie demo tasks", W.cassie_demo_problem, 65536, "standing")
 run("cassie demo + posture (26 rows)", W.cassie_demo_posture_problem, 65536, "standing")
-run("cassie + FrameConstraint", constraint_pb, 65536, "standing")
+run("cassie + FrameConstraint", W.cassie_constraint_problem, 65536, "standing")
 run("cassie CentreOfMassTask", com_pb, 65536, "standing", com=lambda pb: pb.get_centre_of_mass_task())
 prm = ik.pik_parameters(lambdas=[1e-2, 1e-1])
 run("ik::pik demo + posture (2 levels)", W.cassie_demo_posture_problem, 65536, "standing", solve=lambda p, q, t: ik.pik_batch(p, q, t, prm))

@@ -25,8 +25,9 @@ data.cpp:25-58, frame.hpp:37-62,152-182) for a FIXED tree and FIXED frame-task l
 The emitted struct is consumed by dls_spec.cuh (thread-per-problem persistent kernel with lane refill) and -- being
 __host__ __device__ -- by the CPU unit-test harness.  Supported: free-flyer or fixed base; RX/RY/RZ/unaligned
 revolute, continuous and prismatic joints; FrameTask (Position / Orientation / Full, any reference frame), AlignAxisTask,
-PostureTask and CentreOfMassTask (spec kind "com"; the model JSON then carries each joint's "mass" and "com").
-Anything else runs on the generic kernel.
+PostureTask and CentreOfMassTask (spec kind "com"; the model JSON then carries each joint's "mass" and "com"); FrameConstraints
+(spec key "constraints", projected out of the step in step_direction, see gen_project).  Anything else runs on the generic
+kernel.
 """
 import json
 import re
@@ -226,6 +227,33 @@ class Generator:
             for opt in ("arrow_solve", "mirror", "fold_task", "tmem_j", "uniform_solve", "parallel_solve", "presolve", "interleave"):
                 if spec.get(opt) or (opt == "fold_task" and spec.get(opt) is not None):
                     raise ValueError("spec option %r does not support a centre-of-mass task" % opt)
+        # FrameConstraints (frame.hpp:333-465), stacked in insertion order (dls.cpp:26-34): Jc is evaluated by the SOLVER role
+        # with its tasks and projected out of dq in step_direction (gen_project)
+        self.constraints = []
+        crow = 0
+        for cn in spec.get("constraints", []):
+            ktype = {"position": POSITION, "orientation": ORIENTATION, "full": FULL}[cn["type"]]
+            f, ref = self.frames[cn["frame"]], self.frames[cn.get("reference", "universe")]
+            self.constraints.append(dict(frame=f, ref=ref, ktype=ktype, dim=6 if ktype == FULL else 3, row=crow, name=cn["frame"],
+                                         ref_name=cn.get("reference", "universe")))
+            crow += self.constraints[-1]["dim"]
+        if len(self.constraints) > 4 or crow > 12:
+            raise ValueError("at most 4 frame constraints / 12 constraint rows (kMaxConstraints / kMaxConstraintRows)")
+        self.crows = crow
+        self.ucols = []   # velocity columns of Jc that are not structurally zero (U), ascending
+        if self.constraints:
+            # Jc is evaluated and projected by the SOLVER role alone, over columns that are not chain-local
+            for opt in ("arrow_solve", "mirror", "fold_task", "tmem_j", "uniform_solve", "parallel_solve", "presolve", "interleave"):
+                if spec.get(opt) or (opt == "fold_task" and spec.get(opt) is not None):
+                    raise ValueError("spec option %r does not support FrameConstraints" % opt)
+            if any(t["kind"] == "com" for t in self.tasks):
+                raise ValueError("a centre-of-mass task beside FrameConstraints is not supported")
+            cols = set()
+            for cn in self.constraints:
+                cols.update(self.joint_cols(self.constraint_joints(cn))[0])
+            self.ucols = sorted(cols)
+            if len(self.ucols) > 64:
+                raise ValueError("FrameConstraints over more than 64 velocity columns are not supported")
         self.rows = row
         self.tsz = toff
         self.slots = {}  # (row, col) -> slot index
@@ -270,6 +298,156 @@ class Generator:
         """joints whose subtree carries mass: the only ones with centre-of-mass Jacobian columns"""
         ms, _ = self.com_masses()
         return [j for j in range(1, len(self.joints)) if ms[j] > 0]
+
+    # ---- frame constraints ----
+    def support(self, f):
+        """joints that move frame f (its parent joint and that joint's ancestors)"""
+        out, j = set(), f["parent"]
+        while j > 0:
+            out.add(j)
+            j = self.joints[j]["parent"]
+        return out
+
+    def constraint_joints(self, cn):
+        """Joints with non-zero columns in Jc: a joint that moves both the frame and the reference frame adds the same twist
+        to Jf and to rMf.actInv(Jr) (both are its world twist seen from the frame), so its columns cancel."""
+        return sorted(self.support(cn["frame"]) ^ self.support(cn["ref"]))
+
+    def gen_constraints(self, E, world):
+        """FrameConstraint::compute_jacobian (frame.hpp:399-437; iko_constraint_jacobian) of every constraint, unweighted, dense
+        over the columns U at strip slots CSLOT + row * NU + u.  Column c of Jf - rMf.actInv(Jr) is the world twist (v, w) of
+        coordinate c seen from the frame, (Rf^T (v - pf x w), Rf^T w): + for a joint that moves the frame only, - for one
+        that moves the reference frame only, 0 otherwise.  The FK is the role's memoised one."""
+        nu = len(self.ucols)
+        for k, cn in enumerate(self.constraints):
+            E.comment("==== constraint %d: frame %s, %s, reference %s ====" % (k, cn["name"], ["Position", "Orientation", "Full"][cn["ktype"]],
+                                                                           cn["ref_name"]))
+            Rf, pf = self.frame_world(E, cn["frame"], world, "cf")
+            rows = {POSITION: [0, 1, 2], ORIENTATION: [3, 4, 5], FULL: [0, 1, 2, 3, 4, 5]}[cn["ktype"]]
+            own = self.support(cn["frame"])
+            vals = {}   # (constraint row, column) -> value
+
+            def column(col, v, w, sign):
+                if w is None:   # a linear column: w = 0
+                    d, ang = v, [0.0] * 3
+                else:           # v - pf x w
+                    d = [sop(E, [(1.0, v[i]), (pf[(i + 1) % 3], w[(i + 2) % 3], -1), (pf[(i + 2) % 3], w[(i + 1) % 3])], "cd")
+                         for i in range(3)]
+                    ang = [sop(E, [(Rf[3 * k_ + i], w[k_]) for k_ in range(3)], "ca") for i in range(3)]
+                six = [sop(E, [(Rf[3 * k_ + i], d[k_]) for k_ in range(3)], "cl") for i in range(3)] + ang
+                for r, src in enumerate(rows):
+                    vals[(r, col)] = six[src] if sign > 0 else neg(E, six[src], "cn")
+
+            for j in self.constraint_joints(cn):
+                w_, jt = self.fk_joint(E, j, world), self.joints[j]
+                iv, sign = jt["idx_v"], 1 if j in own else -1
+                if jt["type"] == J_FF:   # LOCAL columns: linear along R e_k, angular about R e_k through p
+                    for k_ in range(3):
+                        rk = [w_["R"][k_], w_["R"][3 + k_], w_["R"][6 + k_]]
+                        column(iv + k_, rk, None, sign)
+                        column(iv + 3 + k_, [_cross_comp(E, w_["p"], rk, i, "cv") for i in range(3)], rk, sign)
+                elif jt["type"] in J_REV:
+                    column(iv, [_cross_comp(E, w_["p"], w_["z"], i, "cv") for i in range(3)], w_["z"], sign)
+                else:   # prismatic
+                    column(iv, w_["z"], None, sign)
+            for r in range(cn["dim"]):
+                for u, col in enumerate(self.ucols):   # every slot, zeros too: the QR overwrote them in the last step
+                    E.raw("sJ.set(CSLOT + %d, %s);  // Jc[%d][%d]" % ((cn["row"] + r) * nu + u, lit(vals.get((r, col), 0.0)),
+                                                                    cn["row"] + r, col))
+
+    def gen_project(self):
+        """dq -= W^T (W dq), W an orthonormal basis of the row space of the numerically rank-r part of Jc: the oracle's
+        rank decision (iko_rowspace_projector; rowspace_basis in dls_generic.cuh) on the columns U only.  Householder QR with
+        column pivoting, unrolled over U: the pivot of step k is the first remaining column with the strictly largest
+        squared norm over rows k.. (recomputed every step), a run-time index into the strip; the reflection is applied to
+        every column of U (rows k.. of the columns pivoted earlier are never read again).  r = the number of |R_kk| above
+        eps * min(m, NV) * max |R_kk|; rows 0..r-1 of R, with the columns pivoted before each row set to zero, are
+        orthonormalised by modified Gram-Schmidt, twice.  Steps past |U| would see only zero columns (diagonal 0)."""
+        m, nu = self.crows, len(self.ucols)
+        K = min(m, nu)
+        ind = "        "
+        L = []
+
+        def a(r, u):
+            return "sJ.get(CSLOT + %d)" % (r * nu + u)
+        L.append(ind + "unsigned long long done = 0;   // columns of U pivoted so far")
+        L.append(ind + "int piv[%d];" % K)
+        L.append(ind + "T diag[%d], maxpiv = T(0);" % K)
+        for k in range(K):
+            L.append(ind + "{  // ---- step %d ----" % k)
+            L.append(ind + "    T best = T(-1);")
+            L.append(ind + "    int p = 0;")
+            for u in range(nu):
+                L.append(ind + "    {")
+                L.append(ind + "        T s = T(0);")
+                for r in range(k, m):
+                    L.append(ind + "        { const T x = %s; s += x * x; }" % a(r, u))
+                L.append(ind + "        if (!((done >> %d) & 1ull) && s > best) { best = s; p = %d; }" % (u, u))
+                L.append(ind + "    }")
+            L.append(ind + "    done |= 1ull << p;")
+            L.append(ind + "    piv[%d] = p;" % k)
+            L.append(ind + "    diag[%d] = T(0);" % k)
+            L.append(ind + "    const T nrm = sqrt_(max_(best, T(0)));")
+            L.append(ind + "    if (nrm > T(0)) {")
+            for r in range(k, m):
+                L.append(ind + "        T v%d = sJ.get(CSLOT + %d + p);" % (r, r * nu))
+            L.append(ind + "        v%d -= v%d >= T(0) ? -nrm : nrm;   // v = x - alpha e_k, alpha = -sign(x_k) ||x||" % (k, k))
+            L.append(ind + "        const T vn = %s;" % " + ".join("v%d * v%d" % (r, r) for r in range(k, m)))
+            L.append(ind + "        if (vn > T(0)) {")
+            L.append(ind + "            const T two_over = T(2) / vn;")
+            for u in range(nu):
+                L.append(ind + "            {")
+                for r in range(k, m):
+                    L.append(ind + "                const T a%d = %s;" % (r, a(r, u)))
+                L.append(ind + "                const T s = (%s) * two_over;" % " + ".join("v%d * a%d" % (r, r) for r in range(k, m)))
+                for r in range(k, m):
+                    L.append(ind + "                sJ.set(CSLOT + %d, a%d - s * v%d);" % (r * nu + u, r, r))
+                L.append(ind + "            }")
+            L.append(ind + "        }")
+            L.append(ind + "        diag[%d] = abs_(sJ.get(CSLOT + %d + p));" % (k, k * nu))
+            L.append(ind + "        maxpiv = max_(maxpiv, diag[%d]);" % k)
+            L.append(ind + "    }")
+            L.append(ind + "}")
+        L.append(ind + "const T eps = sizeof(T) == 8 ? T(2.220446049250313e-16) : T(1.1920929e-7);")
+        L.append(ind + "const T thr = eps * T(%d) * maxpiv;   // min(m, nv): the model's nv, not |U|" % min(m, self.nv))
+        L.append(ind + "int rank = 0;")
+        for k in range(K):
+            L.append(ind + "rank += diag[%d] > thr ? 1 : 0;" % k)
+        L.append(ind + "// rows of R: the entries in columns pivoted at earlier steps are zero")
+        for r in range(1, K):
+            for k in range(r):
+                L.append(ind + "sJ.set(CSLOT + %d + piv[%d], T(0));" % (r * nu, k))
+        L.append(ind + "#pragma unroll 1")
+        L.append(ind + "for (int pass = 0; pass < 2; ++pass) {")
+        L.append(ind + "#pragma unroll 1")
+        L.append(ind + "    for (int r = 0; r < rank; ++r) {")
+        L.append(ind + "#pragma unroll 1")
+        L.append(ind + "        for (int p2 = 0; p2 < r; ++p2) {")
+        L.append(ind + "            T s = T(0);")
+        for u in range(nu):
+            L.append(ind + "            s += sJ.get(CSLOT + r * %d + %d) * sJ.get(CSLOT + p2 * %d + %d);" % (nu, u, nu, u))
+        for u in range(nu):
+            L.append(ind + "            sJ.set(CSLOT + r * %d + %d, sJ.get(CSLOT + r * %d + %d) - s * sJ.get(CSLOT + p2 * %d + %d));" % (nu, u, nu, u, nu, u))
+        L.append(ind + "        }")
+        L.append(ind + "        T nr = T(0);")
+        for u in range(nu):
+            L.append(ind + "        { const T x = sJ.get(CSLOT + r * %d + %d); nr += x * x; }" % (nu, u))
+        L.append(ind + "        const T inr = T(1) / sqrt_(nr);")
+        for u in range(nu):
+            L.append(ind + "        sJ.set(CSLOT + r * %d + %d, sJ.get(CSLOT + r * %d + %d) * inr);" % (nu, u, nu, u))
+        L.append(ind + "    }")
+        L.append(ind + "}")
+        L.append(ind + "// dq -= W^T (W dq), one orthonormal row at a time")
+        L.append(ind + "#pragma unroll 1")
+        L.append(ind + "for (int r = 0; r < rank; ++r) {")
+        L.append(ind + "    T s = T(0);")
+        for u, col in enumerate(self.ucols):
+            L.append(ind + "    s += sJ.get(CSLOT + r * %d + %d) * dq[%d];" % (nu, u, col))
+        for u, col in enumerate(self.ucols):
+            L.append(ind + "    dq[%d] -= s * sJ.get(CSLOT + r * %d + %d);" % (col, nu, u))
+        L.append(ind + "}")
+        L.append(ind + "return rank;")
+        return L
 
     # ---- FK of one joint (memoised) ----
     def fk_joint(self, E, j, world):
@@ -412,11 +590,20 @@ class Generator:
         E.lines.extend(body.lines)
         return E.lines
 
-    def gen_evaluate(self, task_ids):
+    def gen_evaluate(self, task_ids, constraints=False):
         """evaluate_w<k>(): FK of the joints supporting the tasks of one warp role, their weighted error rows (-> strip sE)
-        and the non-zero entries of their weighted Jacobian rows (-> strip sJ)."""
+        and the non-zero entries of their weighted Jacobian rows (-> strip sJ); with `constraints` (the SOLVER role) also
+        the constraint Jacobian, on the same FK."""
         E = Emitter()
         world = {}
+        if constraints:
+            for cnt, ti in enumerate(task_ids):
+                if cnt > 0:
+                    E.raw("IKB_PHASE_FENCE();")
+                self.gen_task(E, ti, world)
+            E.raw("IKB_PHASE_FENCE();")
+            self.gen_constraints(E, world)
+            return E.lines
         inter = [g for g in self.spec.get("interleave", []) if all(t in task_ids for t in g)]
         done = set()
         for cnt, ti in enumerate(task_ids):
@@ -1855,11 +2042,12 @@ class Generator:
                     shared[bid] = self.gen_evaluate_mirrored(pair[0], pair[1])
                 evs.append(None)
             else:
-                evs.append(self.gen_evaluate(g))
+                evs.append(self.gen_evaluate(g, constraints=bool(self.constraints) and k == solver))
         self.qmap = None
         dq = self.gen_dq()
         integ = self.gen_integrate()
         rows, nslot = self.rows, len(self.slots)
+        cslot, cslots = nslot, self.crows * len(self.ucols)   # Jc, dense over U, behind the task Jacobian's slots
         # presolve: the solver role factorises the leading block of its own task rows before the first barrier
         P = 0
         self.order = list(range(rows))
@@ -1903,7 +2091,12 @@ class Generator:
         out.append("namespace ikb {")
         out.append("struct %s {" % struct_name)
         out.append("    static constexpr int NQ = %d, NV = %d, M = %d, M0 = %d, TSZ = %d, NSLOT = %d, NFACT = %d;" %
-                   (self.nq, self.nv, rows, self.rows_p0, self.tsz, nslot, nfact))
+                   (self.nq, self.nv, rows, self.rows_p0, self.tsz, nslot + cslots, nfact))
+        if self.constraints:
+            out.append("    // FrameConstraints: MC rows of Jc, dense over the NU velocity columns con_cols(), at strip slots CSLOT + row * NU + u")
+            out.append("    // (written by the SOLVER role's evaluate, factorised in place by project())")
+            out.append("    static constexpr int MC = %d, NU = %d, CSLOT = %d;" % (self.crows, len(self.ucols), cslot))
+            out.append("    static const int *con_cols() { static const int v[] = {%s}; return v; }" % ", ".join(map(str, self.ucols)))
         out.append("    // NQL: configuration registers per thread (arrow specs: a role keeps only the coordinates it reads and steps)")
         out.append("    static constexpr int NQL = %d;" % nql)
         out.append("    // MY: entries of y a role keeps between psolve() and step_role() (arrow specs with the factor in registers: its own rows)")
@@ -2151,10 +2344,20 @@ class Generator:
                 out.append("        if (role == %d) psolve_w%d(sJ, sL, sE, damping2, y, sync);" % (k, k))
             out.append("    }")
         out.append("    // dq = -J^T y from the strip (dls.cpp:52)")
+        if self.constraints:
+            out.append("    // then dq -= W^T (W dq): the null-space projection of the constraints (dls.cpp:26-34,44-52), see gen_project")
         out.append("    template <typename T, typename S>")
         out.append("    static IKB_HD void step_direction(const S &sJ, const T (&y)[M], T (&dq)[NV]) {")
         out.extend(dq)
+        if self.constraints:
+            out.append("        project(sJ, dq);")
         out.append("    }")
+        if self.constraints:
+            out.append("    // W from Jc in the strip (destroyed), dq -= W^T (W dq); returns the numerical rank r of Jc")
+            out.append("    template <typename T, typename S>")
+            out.append("    static IKB_HD int project(const S &sJ, T (&dq)[NV]) {")
+            out.extend(self.gen_project())
+            out.append("    }")
         out.append("    // q <- clamp(integrate(q, step*dq))")
         out.append("    template <typename T>")
         out.append("    static IKB_HD void integrate(T (&q)[NQ], const T (&dq)[NV], T step, const SpecConsts<T, NQ, M> &c) {")
@@ -2287,6 +2490,17 @@ class Generator:
             out.append("    // per joint: mass, then its centre of mass in the joint frame (3) -- the com task's folded constants")
             out.append("    static const double *sig_inertia() { static const double v[] = {%s}; return v; }" %
                        ", ".join(repr(float(x)) for jt in self.joints for x in [jt["mass"]] + list(jt["com"])))
+        if self.constraints:
+            # the constraint list the projection was generated for (dls_spec.cuh spec_has_constraints); emitted only for specs
+            # with constraints
+            out.append("    // FrameConstraints in stacked order: type (0 position, 1 orientation, 2 full), frame and reference frame (parent joint, placement)")
+            out.append("    static constexpr int NCONS = %d;" % len(self.constraints))
+            for nm, vals in (("sig_con_type", [c["ktype"] for c in self.constraints]), ("sig_con_joint", [c["frame"]["parent"] for c in self.constraints]),
+                             ("sig_con_ref_joint", [c["ref"]["parent"] for c in self.constraints])):
+                out.append("    static const int *%s() { static const int v[] = {%s}; return v; }" % (nm, ", ".join(map(str, vals))))
+            for nm, key in (("sig_con_placement", "frame"), ("sig_con_ref_placement", "ref")):
+                out.append("    static const double *%s() { static const double v[] = {%s}; return v; }" %
+                           (nm, ", ".join(repr(float(x)) for c in self.constraints for x in c[key]["placement"])))
         out.append("};")
         out.append("}  // namespace ikb")
         # The Jacobian strip has a type of its own (SJ): the kernel may keep it in tensor memory (TStrip, tmem_scratch.cuh)
